@@ -1,3 +1,4 @@
+import hashlib
 import os
 import sys
 
@@ -22,9 +23,53 @@ def c1():
     return dict(np.load(os.path.join(GOLDEN, "peptide_c1.npz"), allow_pickle=False))
 
 
+KMEANS_CASES = {
+    # name: (n, d, k, rounded to the 1e-4 CSV grid?)
+    "blobs_d2_k5": (3000, 2, 5, False),
+    "blobs_d4_k10_grid": (5000, 4, 10, True),
+    "blobs_d10_k40": (20000, 10, 40, False),
+    "uniform_d3_k7_grid": (4000, 3, 7, True),
+}
+
+
+def kmeans_inputs():
+    """The seeded inputs the reference clustered for kmeans_ref.npz: ``{name}_X`` and ``{name}_init``
+    (its first k rows) for every case of KMEANS_CASES, then ``opt_X`` for the k-means++ and k-search
+    cases, all drawn in this order from one generator."""
+    rng = np.random.default_rng(7)
+    out = {}
+    for name, (n, d, k, grid) in KMEANS_CASES.items():
+        if name.startswith("blobs"):
+            cent = rng.uniform(-0.9, 0.9, size=(k, d))
+            X = cent[rng.integers(0, k, size=n)] + 0.08 * rng.standard_normal((n, d))
+        else:
+            X = rng.uniform(-1, 1, size=(n, d))
+        if grid:
+            X = np.round(X, 4)
+        X = np.ascontiguousarray(X, dtype=np.float64)
+        out[f"{name}_X"], out[f"{name}_init"] = X, X[:k].copy()
+    cent = rng.uniform(-0.8, 0.8, size=(5, 3))
+    out["opt_X"] = np.ascontiguousarray(
+        np.round(cent[rng.integers(0, 5, size=6000)] + 0.09 * rng.standard_normal((6000, 3)), 4))
+    return out
+
+
+def sha256(a: np.ndarray) -> str:
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
 @pytest.fixture(scope="session")
 def kmeans_ref():
-    return dict(np.load(os.path.join(GOLDEN, "kmeans_ref.npz"), allow_pickle=False))
+    """The reference's KMeans outputs (kmeans_ref.npz) with the inputs they were computed from.
+    The inputs are regenerated from their seed rather than stored (the largest is 1.6 MB of
+    incompressible float64); the file keeps each input's SHA-256, so inputs that differ from the
+    ones the reference saw fail here instead of being compared with its outputs."""
+    ref = dict(np.load(os.path.join(GOLDEN, "kmeans_ref.npz"), allow_pickle=False))
+    for key, a in kmeans_inputs().items():
+        if key.endswith("_X"):
+            assert sha256(a) == str(ref[f"{key}_sha256"]), f"regenerated {key} differs from the reference's input"
+        ref[key] = a
+    return ref
 
 
 def synth_features(n, f, seed=0, n_slow=6, dtype=np.float32):

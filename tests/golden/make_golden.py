@@ -15,8 +15,9 @@ Writes (all small, committed):
       the same matrix as a PLUMED colvars text file + feature list, for the step-API tests
       (re-serialised with enough digits to round-trip float32 exactly).
   tests/golden/kmeans_ref.npz     labels / centres produced by the REFERENCE's own
-      ``deep_cartograph.modules.statistics.cluster_data`` (imported from /root/reference,
-      sklearn underneath) on seeded inputs with fixed initial centroids.
+      ``deep_cartograph.modules.statistics.cluster_data`` (sklearn underneath) on seeded inputs
+      with fixed initial centroids; the inputs themselves are kept as SHA-256 digests
+      (tests/conftest.py:kmeans_inputs regenerates them).
 """
 import io
 import json
@@ -87,41 +88,27 @@ def main():
     chk = read_colvars(os.path.join(HERE, "peptide_c1.dat"))[feats].to_numpy(dtype=np.float32)
     assert np.array_equal(chk, X), "text round trip is not exact"
 
-    # KMeans: outputs of the reference's own statistics.cluster_data (sklearn underneath)
+    # KMeans: outputs of the reference's own statistics.cluster_data (sklearn underneath).  The inputs are
+    # not stored: tests/conftest.py regenerates them from their seed and checks them against the digests.
     sys.path.insert(0, REF)
     from deep_cartograph.modules.statistics import cluster_data  # noqa: E402
     import sklearn
+    sys.path.insert(0, os.path.dirname(HERE))
+    from conftest import KMEANS_CASES, kmeans_inputs, sha256  # noqa: E402
     km = {"sklearn_version": np.array(sklearn.__version__)}
-    rng = np.random.default_rng(7)
-    cases = {
-        # name: (n, d, k, rounded to the 1e-4 CSV grid?)
-        "blobs_d2_k5": (3000, 2, 5, False),
-        "blobs_d4_k10_grid": (5000, 4, 10, True),
-        "blobs_d10_k40": (20000, 10, 40, False),
-        "uniform_d3_k7_grid": (4000, 3, 7, True),
-    }
-    for name, (n, d, k, grid) in cases.items():
-        if name.startswith("blobs"):
-            cent = rng.uniform(-0.9, 0.9, size=(k, d))
-            X = cent[rng.integers(0, k, size=n)] + 0.08 * rng.standard_normal((n, d))
-        else:
-            X = rng.uniform(-1, 1, size=(n, d))
-        if grid:
-            X = np.round(X, 4)
-        X = np.ascontiguousarray(X, dtype=np.float64)
-        init = X[:k].copy()
+    inputs = kmeans_inputs()
+    for name in KMEANS_CASES:
+        X, init = inputs[f"{name}_X"], inputs[f"{name}_init"]
         labels, centers = cluster_data(X.copy(), {"algorithm": "kmeans"}, initial_centroids=init.copy())
-        km[f"{name}_X"] = X
-        km[f"{name}_init"] = init
+        km[f"{name}_X_sha256"] = np.array(sha256(X))
         km[f"{name}_labels"] = labels.astype(np.int32)
         km[f"{name}_centers"] = centers
     # ---- the reference's DEFAULT search path: optimize_clustering (k-means++ with random_state=0, three
     # scores per k) and kmeans_clustering without initial centroids, run by the imported reference module
     from deep_cartograph.modules.statistics.statistics import kmeans_clustering, optimize_clustering
-    cent = rng.uniform(-0.8, 0.8, size=(5, 3))
-    Xo = np.ascontiguousarray(np.round(cent[rng.integers(0, 5, size=6000)] + 0.09 * rng.standard_normal((6000, 3)), 4))
+    Xo = inputs["opt_X"]
     lab_o, cen_o = optimize_clustering(Xo.copy(), {"algorithm": "kmeans", "search_interval": [2, 8], "n_init": 3})
-    km["opt_X"], km["opt_labels"], km["opt_centers"] = Xo, lab_o.astype(np.int32), cen_o
+    km["opt_X_sha256"], km["opt_labels"], km["opt_centers"] = np.array(sha256(Xo)), lab_o.astype(np.int32), cen_o
     lab_p, cen_p = kmeans_clustering(Xo.copy(), 6, 4)
     km["pp_labels"], km["pp_centers"] = lab_p.astype(np.int32), cen_p
     from sklearn.metrics import calinski_harabasz_score, davies_bouldin_score, silhouette_score
