@@ -39,9 +39,11 @@
 //      (leader CTA), 2-5 = epilogue (int32 -> FP64: A 2^32 + B 2^24 + C 2^16 is exact in a double,
 //      scaled by 2^-e_i 2^-e_j / (range_i range_j), red.global.add.f64).
 //
-// Error model: only the fixed-point rounding of the inputs remains, |z - z'| <= 2^-23 max|x - c| /
-// range -- the float32 resolution of the data -- unbiased and independent between frames, so its
-// effect on the sums is ~ sqrt(2/M) 2^-23: 1e-10 relative at M = 1e6, against a worst case of 1e-6.
+// Error model: the fixed-point rounding of the inputs, |z - z'| <= 2^-23 max|x - c| / range -- the
+// float32 resolution of the data -- is unbiased and independent between frames, so its effect on the
+// sums is ~ sqrt(2/M) 2^-23: 1e-10 relative at M = 1e6, against a worst case of 1e-6.  The omitted
+// d0 d0 product is a bias: every diagonal entry is low by sum d0^2 ~ 5461 M integer units.
+// tests/test_cov_i8_exact.py holds the outputs to an exact integer model of this arithmetic.
 //
 // Frames are processed in windows (the planes of a window live in the caller's workspace).
 // Roofline: tensor pipe (kind::i8); HBM for the quantise pass (4 + 6 bytes per element).

@@ -190,7 +190,9 @@ def lagged_covariance(X: torch.Tensor, lag: int, mean: Optional[torch.Tensor] = 
     sums (reference cv_calculator.py:2244-2261).
 
     ``xmin`` / ``xmax`` (per-column bounds of X, float32) are used by the exact integer engine
-    (``tc_i8x3``); when absent they are taken from X here (one more pass over X)."""
+    (``tc_i8x3``); when absent they are taken from X here (one more pass over X).  That engine also
+    returns ``clamped`` (int32, device): nonzero if and only if some value of X lay far enough outside
+    the bounds to be clamped to the fixed-point range; the number itself is not a count of values."""
     _need_cuda("X", X, torch.float32)
     n, f, ld = _rows("X", X)
     if not (0 <= lag < n):

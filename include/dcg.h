@@ -122,13 +122,16 @@ int dcg_cov_lag_f32(const float* X, int64_t n_rows, int f, int64_t ld, int lag,
 
 /* ---- A5/A6/A7/A8, exact engine: integer tensor cores ---------------------------------------------
  * Same sums as dcg_cov_lag_f32 (same reference call sites), computed EXACTLY on the int8 tensor
- * cores (tcgen05 kind::i8, int32 accumulation): every value is first rounded to 24-bit fixed point
+ * cores (tcgen05 kind::i8, int32 accumulation): every value is first rounded to 23-bit fixed point
  * relative to its column's range, q = rint((x - mean[j]) * 2^e_j) -- the float32 resolution of the
  * data -- split into three int8 digit planes in the K-major layout of the contraction (one HBM-bound
- * pass), and the planes are contracted by TMA-staged integer MMAs; nothing is rounded afterwards
+ * pass), and the planes are contracted by TMA-staged integer MMAs: the digit products are exact (all
+ * but d0 d0, which is left out), and only the FP64 scaling and adds of the int32 partial sums round
  * (csrc/cov_i8.cu).  `xmin` / `xmax` (f, float32, device): per-column bounds of X over ALL n_rows rows
- * (the column statistics, dcg_colstats_f32); values outside them are clamped and counted in
- * `info[0]` (int32, device, may be NULL).  The digit planes of a window of frames live in `ws`.     */
+ * (the column statistics, dcg_colstats_f32); values outside them may be clamped to |q| <= 4161536.
+ * `info[0]` (int32, device, may be NULL) is nonzero if and only if some value was clamped; its value
+ * counts groups of values and depends on the kernel path.  The digit planes of a window of frames live
+ * in `ws`.                                                                                            */
 #define DCG_COV_TC_I8X3    4 /* tcgen05 kind::i8 on three int8 digit planes: exact accumulation    */
 size_t dcg_cov_i8_workspace_bytes(int64_t n_rows, int f, int lag, int block);
 int dcg_cov_lag_i8_f32(const float* X, int64_t n_rows, int f, int64_t ld, int lag,
