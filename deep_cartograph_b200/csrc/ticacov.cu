@@ -378,11 +378,15 @@ gen_eig_small_kernel(const double* __restrict__ Hm, const double* __restrict__ G
       }
   }
   if (lane < b) {
+    // rank by value, ties by index: a permutation only if every key compares, so NaN (a pencil that is not
+    // definite, e.g. from a failed factorisation upstream; flagged through the residuals) ranks as -inf --
+    // otherwise ranks collide and order[] keeps unwritten slots that index V below
     const double mine = A[lane][lane];
+    const double km = (mine == mine) ? mine : -INFINITY;
     int r = 0;
     for (int j = 0; j < b; ++j) {
-      const double o = A[j][j];
-      r += (o > mine) || (o == mine && j < lane);
+      const double o = (A[j][j] == A[j][j]) ? A[j][j] : -INFINITY;
+      r += (o > km) || (o == km && j < lane);
     }
     order[r] = lane;
     theta[(size_t)blockIdx.x * b + r] = mine;
