@@ -24,6 +24,7 @@ COV_ENGINES = {"simt_f32": COV_SIMT_F32, "tc_3xtf32": COV_TC_3XTF32, "tc_1xtf32"
                "tc_3xf16": COV_TC_3XF16, "tc_i8x3": COV_TC_I8X3}
 
 LINKAGE_METHODS = {"single": 0, "complete": 1, "average": 2, "ward": 3}   # DCG_LINK_* (dcg.h)
+HDBSCAN_MAX_MIN_SAMPLES = 64                                              # DCG_HDBSCAN_MAX_MIN_SAMPLES (dcg.h)
 
 _SIGNATURES = {
     # name: (restype, [argtypes])
@@ -77,6 +78,9 @@ _SIGNATURES = {
     "dcg_cluster_dispersion": (_c_int, [_p, _c_i64, _c_int, _c_i64, _c_int, _p, _p, _c_int, _p, _p, _p]),
     "dcg_linkage_workspace_bytes": (_c_sz, [_c_i64, _c_int, _c_int]),
     "dcg_linkage_f64": (_c_int, [_p, _c_i64, _c_int, _c_i64, _c_int, _p, _p, _c_sz, _p]),
+    "dcg_hdbscan_workspace_bytes": (_c_sz, [_c_i64, _c_int, _c_int]),
+    "dcg_core_distances_f64": (_c_int, [_p, _c_i64, _c_int, _c_i64, _c_int, _p, _p, _c_sz, _p]),
+    "dcg_mreach_mst_f64": (_c_int, [_p, _c_i64, _c_int, _c_i64, _p, _p, _p, _c_sz, _p]),
     "dcg_fes_bin_f32": (_c_int, [_p, _c_i64, _c_i64, _c_int, _c_int, C.c_double, C.c_double, C.c_double, C.c_double,
                                  _c_int, _c_int, _p, _p, _p]),
     "dcg_fes_smooth_f64": (_c_int, [_p, _c_int, _c_int, _c_int, C.c_double, C.c_double, C.c_double, _p, _p, _p, _p]),

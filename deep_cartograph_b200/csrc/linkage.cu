@@ -19,6 +19,14 @@
 // Finish (both): a stable sort of the merges by distance (numpy mergesort semantics: a rank sort on the
 // unique key (distance, merge index)), then the relabelling pass on one thread: scipy's `label`
 // (union-find, smaller root first) or sklearn's `_single_linkage_label` (no swap).
+//
+// HDBSCAN (sklearn.cluster.HDBSCAN, algorithm "auto" on dense Euclidean data = _hdbscan_prims), O(n) memory:
+//   4. core_dist_kernel      core[i] = distance from frame i to its min_samples-th nearest frame (itself
+//                            included, at 0): a brute-force k-smallest selection with the arithmetic above.
+//   3. prim_kernel           with `core` set: sklearn's mst_from_data_matrix, Prim from node 0 on the
+//                            mutual-reachability distance max(core[c], core[j], dist(c, j)); each edge is
+//                            recorded from the tree node that last strictly improved the new node.
+// The edge sort (numpy's default argsort, not stable) and the union-find stay on the host.
 #include <cooperative_groups.h>
 #include <math_constants.h>
 #include <climits>
@@ -245,12 +253,17 @@ nn_chain_kernel(double* __restrict__ D, int n, int64_t ldD, int method, double* 
   cl.sync();    // no CTA leaves while a peer may still read its partials
 }
 
-// ---- 3. Prim (single) -------------------------------------------------------------------------------------
-// cur: n doubles (distance of every frame to the tree, -1 once in the tree; each CTA touches its strip only);
-// zraw rows (current node, new node, distance, 0) in visiting order; phases[0] = steps.
+// ---- 3. Prim (single; HDBSCAN's mutual-reachability MST when core != nullptr) ---------------------------------
+// cur: n doubles (distance of every frame to the tree, -1 once in the tree; each CTA touches its strip only).
+// core == nullptr: zraw rows of 4, (current node, new node, distance, 0), in visiting order (mst_linkage_core).
+// core set: src (n ints) holds the tree node that last strictly improved each frame (sklearn's
+//   current_sources); zraw rows of 3, (src[new], new, distance), in visiting order (mst_from_data_matrix).
+//   The CTA that owns the new node writes its row, so src is only ever read by the CTA that wrote it.
+// phases[0] = phases[1] = steps.
 __global__ void __launch_bounds__(kThreads, 1)
-prim_kernel(const double* __restrict__ Y, int n, int d, int64_t ld, int stage, double* __restrict__ cur,
-            double* __restrict__ zraw, long long* __restrict__ phases) {
+prim_kernel(const double* __restrict__ Y, int n, int d, int64_t ld, int stage, const double* __restrict__ core,
+            double* __restrict__ cur, int* __restrict__ src, double* __restrict__ zraw,
+            long long* __restrict__ phases) {
   extern __shared__ double ysm[];
   cg::cluster_group cl = cg::this_cluster();
   const int rank = (int)cl.block_rank();
@@ -271,12 +284,15 @@ prim_kernel(const double* __restrict__ Y, int n, int d, int64_t ld, int stage, d
     ys_ld = d;
   }
   for (int j = lo + tid; j < hi; j += kThreads) cur[j] = CUDART_INF;
+  if (core)
+    for (int j = lo + tid; j < hi; j += kThreads) src[j] = 1;     // sklearn's np.ones; every frame is set before use
   if (tid == 0) s_cur = 0;
   int par = 0;
   __syncthreads();
   for (int step = 0; step < n - 1; ++step) {
     const int c = s_cur;
     const double* yc = Y + (int64_t)c * ld;
+    const double core_c = core ? core[c] : 0.0;
     double bv = CUDART_INF;
     int bi = INT_MAX;
     for (int j = lo + tid; j < hi; j += kThreads) {
@@ -289,8 +305,17 @@ prim_kernel(const double* __restrict__ Y, int n, int d, int64_t ld, int stage, d
         const double t = __dsub_rn(__ldg(yc + f), yj[f]);
         s = __dadd_rn(s, __dmul_rn(t, t));
       }
-      const double left = __dsqrt_rn(s);
-      if (left < cj) { cj = left; cur[j] = cj; }
+      double left = __dsqrt_rn(s);
+      if (core) {                                   // Cython's max(core_c, core_j, dist): first of the largest
+        double m = core_c;
+        const double cj_core = core[j];
+        if (cj_core > m) m = cj_core;
+        if (left > m) m = left;
+        left = m;
+        if (left < cj) { cj = left; cur[j] = cj; src[j] = c; }
+      } else if (left < cj) {
+        cj = left; cur[j] = cj;
+      }
       if (cj < bv) { bv = cj; bi = j; }
     }
     cta_argmin(bv, bi, red);
@@ -300,9 +325,12 @@ prim_kernel(const double* __restrict__ Y, int n, int d, int64_t ld, int stage, d
       const Part q = cluster_argmin(cl, &part[par]);
       if (tid == 0) {
         const int nxt = q.i == INT_MAX ? 0 : q.i;
-        if (rank == 0) {
+        if (!core && rank == 0) {
           double* z = zraw + (size_t)4 * step;
           z[0] = (double)c; z[1] = (double)nxt; z[2] = q.v; z[3] = 0.0;
+        } else if (core && nxt >= lo && nxt < hi) {
+          double* z = zraw + (size_t)3 * step;
+          z[0] = (double)src[nxt]; z[1] = (double)nxt; z[2] = q.v;
         }
         s_cur = nxt;
       }
@@ -312,6 +340,78 @@ prim_kernel(const double* __restrict__ Y, int n, int d, int64_t ld, int stage, d
   }
   if (rank == 0 && tid == 0) { phases[0] = n - 1; phases[1] = n - 1; }
   cl.sync();    // no CTA leaves while a peer may still read its partials
+}
+
+// ---- 4. HDBSCAN core distances ------------------------------------------------------------------------------
+// One warp per query frame, kCoreWarps queries per CTA.  The CTA stages `rows` candidate frames at a time in
+// shared memory (row stride lds, odd, so the lanes' 8-byte reads hit distinct banks); lane l scans the tile
+// rows l, l + 32, ... and keeps the k smallest squared distances it has seen in a register list of KC >= k
+// slots, ascending.  The KC - k bottom slots hold -1 (below every squared distance) and never move, so the
+// top slot is the lane's k-th smallest and rejects any candidate that is not below it.  The 32 lane lists
+// are then merged by k warp-wide pops of the smallest head; the k-th pop is the query's k-th smallest.
+// Only the value is used, so ties among neighbours do not matter.
+constexpr int kCoreWarps = 8;
+constexpr int kCoreTileDoubles = 6144;          // 48 KB of candidate rows per stage
+
+template <int KC>
+__device__ __forceinline__ void topk_insert(double (&lst)[KC], double v) {
+#pragma unroll
+  for (int t = KC - 1; t > 0; --t) lst[t] = v < lst[t - 1] ? lst[t - 1] : (v < lst[t] ? v : lst[t]);
+  lst[0] = v < lst[0] ? v : lst[0];
+}
+
+template <int KC>
+__global__ void __launch_bounds__(kCoreWarps * 32)
+core_dist_kernel(const double* __restrict__ Y, int n, int d, int64_t ld, int k, int rows, int lds,
+                 double* __restrict__ core) {
+  extern __shared__ double tile[];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int q = blockIdx.x * kCoreWarps + warp;
+  const double* yq = Y + (int64_t)min(q, n - 1) * ld;
+  double lst[KC];
+#pragma unroll
+  for (int t = 0; t < KC; ++t) lst[t] = t < KC - k ? -1.0 : CUDART_INF;
+  for (int j0 = 0; j0 < n; j0 += rows) {
+    const int cnt = min(rows, n - j0);
+    __syncthreads();
+    for (int e = threadIdx.x; e < cnt * d; e += kCoreWarps * 32) {
+      const int r = e / d, f = e % d;
+      tile[r * lds + f] = Y[(int64_t)(j0 + r) * ld + f];
+    }
+    __syncthreads();
+    for (int r = lane; r < cnt; r += 32) {
+      const double* yj = tile + r * lds;
+      double s = 0.0;
+      for (int f = 0; f < d; ++f) {
+        const double t = __dsub_rn(__ldg(yq + f), yj[f]);
+        s = __dadd_rn(s, __dmul_rn(t, t));
+      }
+      if (s < lst[KC - 1]) topk_insert(lst, s);
+    }
+  }
+  double kth = 0.0;
+  for (int p = 0; p < k; ++p) {
+    double head = CUDART_INF;
+#pragma unroll
+    for (int t = KC - 1; t >= 0; --t)
+      if (lst[t] >= 0.0) head = lst[t];
+    double best = head;
+    int who = lane;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const double ob = __shfl_xor_sync(0xffffffffu, best, o);
+      const int ow = __shfl_xor_sync(0xffffffffu, who, o);
+      if (ob < best || (ob == best && ow < who)) { best = ob; who = ow; }
+    }
+    kth = best;
+    if (who == lane) {
+      bool done = false;
+#pragma unroll
+      for (int t = 0; t < KC; ++t)
+        if (!done && lst[t] >= 0.0) { lst[t] = -1.0; done = true; }
+    }
+  }
+  if (lane == 0 && q < n) core[q] = __dsqrt_rn(kth);
 }
 
 // ---- finish: stable sort by distance + relabelling --------------------------------------------------------
@@ -392,6 +492,26 @@ bool link_layout(int64_t n, int method, LinkLayout& L) {
 
 bool valid_method(int m) { return m >= DCG_LINK_SINGLE && m <= DCG_LINK_WARD; }
 
+// HDBSCAN: step counters, the Prim distances to the tree and the Prim edge sources.
+struct HdbLayout { size_t phases, cur, src, total; };
+
+bool hdb_layout(int64_t n, HdbLayout& L) {
+  if (n < 2 || n > (INT_MAX - 1) / 2) return false;
+  size_t o = 0;
+  auto take_bytes = [&](size_t bytes) { const size_t at = o; o = align_up(o + bytes, 256); return at; };
+  L.phases = take_bytes(2 * sizeof(long long));
+  L.cur = take_bytes((size_t)n * sizeof(double));
+  L.src = take_bytes((size_t)n * sizeof(int));
+  L.total = o;
+  return true;
+}
+
+int core_tile_rows(int d, int& lds) {
+  lds = d | 1;
+  const int rows = kCoreTileDoubles / lds;
+  return rows >= 32 ? rows / 32 * 32 : max(rows, 1);
+}
+
 template <typename... KArgs, typename... Args>
 cudaError_t launch_cluster(void (*kernel)(KArgs...), size_t smem, cudaStream_t st, Args... args) {
   cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
@@ -444,7 +564,7 @@ extern "C" int dcg_linkage_f64(const double* Y, int64_t n, int d, int64_t ld, in
     const size_t stage_bytes = (size_t)s * d * sizeof(double);
     const int stage = stage_bytes <= kPrimStageBytes;
     DCG_CUDA_TRY(launch_cluster(prim_kernel, stage ? stage_bytes : 0, st, Y, ni, d, ld, stage,
-                                (double*)(w + L.cur), zraw, phases));
+                                (const double*)nullptr, (double*)(w + L.cur), (int*)nullptr, zraw, phases));
   } else {
     double* D = (double*)(w + L.D);
     const dim3 grid((unsigned)ceil_div(L.ldD, kDistTile), (unsigned)ceil_div(n, kDistTile));
@@ -457,5 +577,55 @@ extern "C" int dcg_linkage_f64(const double* Y, int64_t n, int d, int64_t ld, in
   linkage_label_kernel<<<1, 1024, 0, st>>>(Z, ni, (int*)(w + L.parent), (int*)(w + L.usize),
                                            method != DCG_LINK_SINGLE, phases);
   DCG_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" size_t dcg_hdbscan_workspace_bytes(int64_t n, int d, int min_samples) {
+  HdbLayout L;
+  if (d < 1 || min_samples < 1 || min_samples > DCG_HDBSCAN_MAX_MIN_SAMPLES || min_samples > n ||
+      !hdb_layout(n, L))
+    return 0;
+  return L.total;
+}
+
+extern "C" int dcg_core_distances_f64(const double* Y, int64_t n, int d, int64_t ld, int min_samples, double* core,
+                                      void* ws, size_t ws_bytes, void* stream) {
+  (void)ws; (void)ws_bytes;           // no workspace today; the argument keeps the HDBSCAN entry points alike
+  if (n < 2 || n > (INT_MAX - 1) / 2 || d < 1 || ld < d) return DCG_E_SHAPE;
+  if (min_samples < 1 || min_samples > DCG_HDBSCAN_MAX_MIN_SAMPLES || min_samples > n) return DCG_E_SHAPE;
+  if (!Y || !core) return DCG_E_NULL;
+  int lds;
+  const int rows = core_tile_rows(d, lds);
+  const size_t smem = (size_t)rows * lds * sizeof(double);
+  if (smem > kPrimStageBytes) return DCG_E_SHAPE;
+  cudaStream_t st = (cudaStream_t)stream;
+  const unsigned grid = (unsigned)ceil_div(n, kCoreWarps);
+  const int ni = (int)n;
+  auto run = [&](auto kernel) -> int {
+    DCG_CUDA_TRY(ensure_dynamic_smem((const void*)kernel, smem));
+    kernel<<<grid, kCoreWarps * 32, smem, st>>>(Y, ni, d, ld, min_samples, rows, lds, core);
+    DCG_LAUNCH_CHECK();
+    return 0;
+  };
+  if (min_samples <= 8) return run(core_dist_kernel<8>);
+  if (min_samples <= 16) return run(core_dist_kernel<16>);
+  if (min_samples <= 32) return run(core_dist_kernel<32>);
+  return run(core_dist_kernel<64>);
+}
+
+extern "C" int dcg_mreach_mst_f64(const double* Y, int64_t n, int d, int64_t ld, const double* core, double* mst,
+                                  void* ws, size_t ws_bytes, void* stream) {
+  HdbLayout L;
+  if (n < 2 || n > (INT_MAX - 1) / 2 || d < 1 || ld < d) return DCG_E_SHAPE;
+  hdb_layout(n, L);
+  if (!Y || !core || !mst) return DCG_E_NULL;
+  if (!ws || ws_bytes < L.total) return DCG_E_WORKSPACE;
+  char* w = (char*)ws;
+  const int ni = (int)n;
+  const int s = (ni + kCtas - 1) / kCtas;
+  const size_t stage_bytes = (size_t)s * d * sizeof(double);
+  const int stage = stage_bytes <= kPrimStageBytes;
+  DCG_CUDA_TRY(launch_cluster(prim_kernel, stage ? stage_bytes : 0, (cudaStream_t)stream, Y, ni, d, ld, stage,
+                              core, (double*)(w + L.cur), (int*)(w + L.src), mst, (long long*)(w + L.phases)));
   return 0;
 }

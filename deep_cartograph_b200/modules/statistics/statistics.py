@@ -15,8 +15,13 @@ that labels from fixed initial centroids are identical to the reference's:
 Agglomerative clustering (reference ``hierarchical_clustering``, :285) runs on the device when
 ``settings["backend"]["hierarchical_on_device"]`` is true: ``linkage_tree`` builds the same merge tree as
 scikit-learn (``ops.linkage``, csrc/linkage.cu), ``cut_tree`` restates sklearn's ``_hc_cut``, and
-``optimize_clustering`` builds the tree once and cuts it for every k.  Without the flag, and for HDBSCAN,
-the algorithm is reported as outside the hot path and the step exits.
+``optimize_clustering`` builds the tree once and cuts it for every k.
+
+HDBSCAN runs on the device when ``settings["backend"]["hdbscan_on_device"]`` is true: ``hdbscan_tree``
+builds sklearn's single-linkage tree from device core distances and a device mutual-reachability MST
+(``ops.core_distances``, ``ops.mreach_mst``) in O(N) memory, and ``hdbscan_labels`` restates sklearn's
+``tree_to_labels``.  Without its flag, either algorithm is reported as outside the hot path and the step
+exits.
 """
 from __future__ import annotations
 
@@ -263,6 +268,8 @@ def cluster_data(features, settings: Dict, initial_centroids=None) -> Tuple[np.n
         return kmeans_clustering(features, settings["num_clusters"], settings["n_init"], initial_centroids)
     if settings["algorithm"] == "hierarchical" and _hierarchical_on_device(settings):
         return hierarchical_clustering(features, settings["num_clusters"], settings.get("linkage", "complete"))
+    if settings["algorithm"] == "hdbscan" and _hdbscan_on_device(settings):
+        return hdbscan_clustering(features, settings)
     if settings["algorithm"] in ("hdbscan", "hierarchical"):
         _outside_hot_path(settings["algorithm"])
     raise Exception(f"clustering algorithm {settings['algorithm']} not implemented")
@@ -340,9 +347,17 @@ def optimize_clustering(features, settings: Dict):
     the interval and the best k maximises (CH - DB + silhouette) / 3.  Like the reference it mutates
     ``settings['num_clusters']`` and ignores ``opt_num_clusters``.  The silhouette is exact up to
     ``settings['silhouette_max_samples']`` frames (default 50000, O(N^2) on the device); beyond that it is
-    sklearn's ``sample_size`` estimator on that many frames (seed 0) and a warning says so."""
+    sklearn's ``sample_size`` estimator on that many frames (seed 0) and a warning says so.
+    HDBSCAN (with ``backend.hdbscan_on_device``) takes no number of clusters: it runs once, unscored."""
     algorithm = settings.get("algorithm", "kmeans")
     tree = None
+    if algorithm == "hdbscan" and _hdbscan_on_device(settings):
+        logger.info("HDBSCAN finds the number of clusters itself: the search over search_interval and its "
+                    "scores are skipped")
+        labels, centroids = hdbscan_clustering(features, settings)
+        if len(centroids) == 0:
+            logger.warning("No clusters found using the provided settings. Try different settings or a different algorithm")
+        return labels, centroids
     if algorithm == "hierarchical" and _hierarchical_on_device(settings):
         tree = linkage_tree(features, settings.get("linkage", "complete"))     # one tree, cut for every k
     elif algorithm != "kmeans":
@@ -446,12 +461,255 @@ def hierarchical_clustering(feature_matrix, num_clusters: int, linkage: str = "c
     return labels, _member_means(feats, labels, num_clusters)
 
 
+# ---- HDBSCAN ------------------------------------------------------------------------------------------------
+# sklearn.cluster.HDBSCAN (scikit-learn 1.9.0, sklearn/cluster/_hdbscan/) with metric="euclidean" and
+# algorithm="auto" on dense finite data: _hdbscan_prims, then tree_to_labels with allow_single_cluster=False.
+HIERARCHY_DTYPE = np.dtype([("left_node", np.intp), ("right_node", np.intp), ("value", np.float64),
+                            ("cluster_size", np.intp)])      # sklearn's HIERARCHY_dtype (_tree.pyx)
+
+
+def _hdbscan_on_device(settings: Dict) -> bool:
+    return bool((settings.get("backend") or {}).get("hdbscan_on_device", False))
+
+
+def single_linkage_from_mst(mst) -> np.ndarray:
+    """sklearn's ``_process_mst`` (hdbscan.py) on the (n-1) x 3 rows (source, new node, distance) of
+    ``ops.mreach_mst`` in Prim order: the rows are reordered by numpy's default ``argsort`` of the
+    distances -- not stable, so the tie order is numpy's own and this must stay a numpy argsort on the
+    host -- and ``make_single_linkage`` (_linkage.pyx) merges them with sklearn's ``UnionFind``
+    (_hierarchical_fast.pyx): merge i creates node n + i, whose children are the roots of the two
+    endpoints, left first.  Returns the HIERARCHY_DTYPE tree."""
+    mst = np.asarray(mst, dtype=np.float64)
+    n = mst.shape[0] + 1
+    mst = mst[np.argsort(mst[:, 2])]
+    a = mst[:, 0].astype(np.intp).tolist()
+    b = mst[:, 1].astype(np.intp).tolist()
+    parent = [-1] * (2 * n - 1)
+    size = [1] * n + [0] * (n - 1)
+    left, right, csize = [0] * (n - 1), [0] * (n - 1), [0] * (n - 1)
+
+    def find(x):
+        r = x
+        while parent[r] != -1:
+            r = parent[r]
+        while x != r and parent[x] != r:          # path compression (does not change any root)
+            parent[x], x = r, parent[x]
+        return r
+
+    for i in range(n - 1):
+        ra, rb = find(a[i]), find(b[i])
+        left[i], right[i] = ra, rb
+        csize[i] = size[ra] + size[rb]
+        parent[ra] = parent[rb] = n + i
+        size[n + i] = csize[i]
+    tree = np.empty(n - 1, dtype=HIERARCHY_DTYPE)
+    tree["left_node"], tree["right_node"], tree["value"], tree["cluster_size"] = left, right, mst[:, 2], csize
+    return tree
+
+
+def hdbscan_tree(features, min_samples: int) -> np.ndarray:
+    """sklearn ``HDBSCAN(min_samples=min_samples)._single_linkage_tree_`` (``_hdbscan_prims``): core
+    distances and the mutual-reachability MST on the device (``ops.core_distances``, ``ops.mreach_mst``),
+    then ``single_linkage_from_mst`` on the host.  O(N) memory."""
+    Y = _to_device(features)
+    return single_linkage_from_mst(ops.mreach_mst(Y, ops.core_distances(Y, min_samples)).cpu().numpy())
+
+
+def _bfs_hierarchy(left, right, n: int, root: int) -> List[int]:
+    """``bfs_from_hierarchy`` (_tree.pyx): the nodes under ``root`` level by level, left before right."""
+    out, queue = [], [root]
+    while queue:
+        out.extend(queue)
+        nxt = []
+        for x in queue:
+            if x >= n:
+                nxt.append(left[x - n])
+                nxt.append(right[x - n])
+        queue = nxt
+    return out
+
+
+def _condense_tree(tree: np.ndarray, min_cluster_size: int):
+    """``_condense_tree`` (_tree.pyx): rows (parent, child, lambda, child size) in sklearn's row order, as
+    four numpy arrays."""
+    left, right = tree["left_node"].tolist(), tree["right_node"].tolist()
+    value, size = tree["value"].tolist(), tree["cluster_size"].tolist()
+    n = len(left) + 1
+    root = 2 * (n - 1)
+    next_label = n + 1
+    relabel = [0] * (root + 1)
+    relabel[root] = n
+    ignore = bytearray(root + 1)
+    rows = []
+    for node in _bfs_hierarchy(left, right, n, root):
+        if ignore[node] or node < n:
+            continue
+        l, r, dist = left[node - n], right[node - n], value[node - n]
+        lam = 1.0 / dist if dist > 0.0 else np.inf
+        lc = size[l - n] if l >= n else 1
+        rc = size[r - n] if r >= n else 1
+        if lc >= min_cluster_size and rc >= min_cluster_size:
+            relabel[l] = next_label
+            next_label += 1
+            rows.append((relabel[node], relabel[l], lam, lc))
+            relabel[r] = next_label
+            next_label += 1
+            rows.append((relabel[node], relabel[r], lam, rc))
+            continue
+        if lc < min_cluster_size and rc < min_cluster_size:
+            fall = (l, r)
+        elif lc < min_cluster_size:
+            relabel[r] = relabel[node]
+            fall = (l,)
+        else:
+            relabel[l] = relabel[node]
+            fall = (r,)
+        for sub in fall:
+            for sub_node in _bfs_hierarchy(left, right, n, sub):
+                if sub_node < n:
+                    rows.append((relabel[node], sub_node, lam, 1))
+                ignore[sub_node] = 1
+    parent, child, lam, csize = zip(*rows)
+    return (np.array(parent, dtype=np.intp), np.array(child, dtype=np.intp), np.array(lam, dtype=np.float64),
+            np.array(csize, dtype=np.intp))
+
+
+def hdbscan_labels(tree, min_cluster_size: int = 5, cluster_selection_method: str = "eom",
+                   cluster_selection_epsilon: float = 0.0, max_cluster_size: Optional[int] = None) -> np.ndarray:
+    """sklearn's ``tree_to_labels`` (sklearn/cluster/_hdbscan/_tree.pyx) with ``allow_single_cluster=False``,
+    restated in numpy: condense the single-linkage ``tree`` (HIERARCHY_DTYPE) at ``min_cluster_size``,
+    compute the stabilities, select clusters by ``eom`` (excess of mass, capped at ``max_cluster_size``) or
+    ``leaf``, merge them upwards to ``cluster_selection_epsilon``, and label each frame with its selected
+    cluster (numbered in increasing condensed-node order) or -1 for noise.  Every tie-breaking detail is
+    sklearn's: the summation order of the stabilities and the iteration order of its Python sets."""
+    if int(min_cluster_size) < 2:
+        raise ValueError(f"min_cluster_size must be at least 2, got {min_cluster_size}")
+    if cluster_selection_method not in ("eom", "leaf"):
+        raise ValueError(f"cluster_selection_method must be 'eom' or 'leaf', got {cluster_selection_method!r}")
+    tree = np.asarray(tree)
+    parent, child, lam, csize = _condense_tree(tree, int(min_cluster_size))
+    eps = float(cluster_selection_epsilon)
+    # _compute_stability: sum of (lambda - birth(parent)) * size over the rows, in row order
+    root = int(parent.min())
+    births = np.full(max(int(child.max()), root) + 1, np.nan)
+    births[child] = lam
+    births[root] = 0.0
+    stab_arr = np.zeros(int(parent.max()) - root + 1)
+    np.add.at(stab_arr, parent - root, (lam - births[parent]) * csize.astype(np.float64))
+    stability = {root + i: v for i, v in enumerate(stab_arr.tolist())}
+    # _get_clusters
+    node_list = sorted(stability.keys(), reverse=True)[:-1]
+    ct = csize > 1                                                       # the cluster tree's rows
+    ct_parent, ct_child, ct_lam = parent[ct].tolist(), child[ct].tolist(), lam[ct].tolist()
+    children: Dict[int, List[int]] = {}
+    row_of: Dict[int, int] = {}
+    for i, (p_, c_) in enumerate(zip(ct_parent, ct_child)):
+        children.setdefault(p_, []).append(c_)
+        row_of[c_] = i
+    cluster_sizes = dict(zip(ct_child, csize[ct].tolist()))
+    n_samples = int(child[csize == 1].max()) + 1
+    if max_cluster_size is None:
+        max_cluster_size = n_samples + 1
+    is_cluster = {c: True for c in node_list}
+
+    def below(node):                                                     # bfs_from_cluster_tree, node excluded
+        out, queue = [], list(children.get(node, ()))
+        while queue:
+            out.extend(queue)
+            queue = [c for q in queue for c in children.get(q, ())]
+        return out
+
+    def epsilon_search(leaves):
+        selected, processed = [], set()
+        for leaf in leaves:
+            if 1 / ct_lam[row_of[leaf]] < eps:
+                if leaf not in processed:
+                    node = leaf                                          # traverse_upwards
+                    while True:
+                        up = ct_parent[row_of[node]]
+                        if up == root or 1 / ct_lam[row_of[up]] > eps:
+                            top = node if up == root else up
+                            break
+                        node = up
+                    selected.append(top)
+                    processed.update(below(top))
+            else:
+                selected.append(leaf)
+        return set(selected)
+
+    if cluster_selection_method == "eom":
+        for node in node_list:
+            sub = np.sum([stability[c] for c in children.get(node, ())])
+            if sub > stability[node] or cluster_sizes[node] > max_cluster_size:
+                is_cluster[node] = False
+                stability[node] = sub
+            else:
+                for sub_node in below(node):
+                    is_cluster[sub_node] = False
+        if eps != 0.0 and ct_parent:
+            eom_clusters = [c for c in is_cluster if is_cluster[c]]
+            if len(eom_clusters) == 1 and eom_clusters[0] == min(ct_parent):
+                selected = []
+            else:
+                selected = epsilon_search(set(eom_clusters))
+            for c in is_cluster:
+                is_cluster[c] = c in selected
+    else:
+        leaves = []                                                      # get_cluster_tree_leaves: DFS order
+        if ct_parent:
+            stack = [min(ct_parent)]
+            while stack:
+                node = stack.pop()
+                kids = children.get(node)
+                if kids:
+                    stack.extend(reversed(kids))
+                else:
+                    leaves.append(node)
+        leaves = set(leaves)
+        selected = epsilon_search(leaves) if eps != 0.0 else leaves
+        for c in is_cluster:
+            is_cluster[c] = c in selected
+    clusters = sorted(c for c in is_cluster if is_cluster[c])
+    # _do_labelling: a frame's label is that of its nearest selected ancestor; none below the root is noise.
+    # Condensed node ids grow from parent to child, so one increasing pass resolves every node.
+    label_of = np.full(int(parent.max()) + 1, -1, dtype=np.intp)
+    label_of[clusters] = np.arange(len(clusters))
+    up_of = np.empty(int(parent.max()) + 1, dtype=np.intp)
+    up_of[child[child >= root]] = parent[child >= root]
+    for c in range(root + 1, int(parent.max()) + 1):
+        if label_of[c] < 0:
+            label_of[c] = label_of[up_of[c]]
+    pts = child < root
+    labels = np.empty(root, dtype=np.intp)
+    labels[child[pts]] = label_of[parent[pts]]
+    return labels
+
+
+def hdbscan_clustering(feature_matrix, settings: Dict) -> Tuple[np.ndarray, np.ndarray]:
+    """``HDBSCAN(min_cluster_size, min_samples, cluster_selection_epsilon, max_cluster_size,
+    cluster_selection_method).fit_predict`` with the schema's values, the tree built on the device, and
+    the FP64 member means of clusters 0..K-1 as centroids (noise, -1, excluded).  The centroid rule is the
+    one the reference applies to hierarchical clustering (statistics.py:330-335); its own HDBSCAN wrapper is
+    assumed to do the same.  ``min_samples`` None means ``min_cluster_size``, as in scikit-learn."""
+    logger.debug("Clustering frames with HDBSCAN...")
+    feats = np.asarray(feature_matrix)
+    mcs = int(settings.get("min_cluster_size", 5))
+    ms = settings.get("min_samples")
+    tree = hdbscan_tree(feats, mcs if ms is None else int(ms))
+    labels = hdbscan_labels(tree, mcs, settings.get("cluster_selection_method", "eom"),
+                            settings.get("cluster_selection_epsilon", 0.0), settings.get("max_cluster_size"))
+    k = int(labels.max()) + 1
+    means = _member_means(feats, labels, k) if k > 0 else np.empty((0, feats.shape[1]))
+    return labels, means
+
+
 def _outside_hot_path(algorithm):
-    """hdbscan, and hierarchical clustering without ``backend.hierarchical_on_device``, are not part of the
+    """hierarchical clustering and hdbscan without their ``backend.*_on_device`` flag are not part of the
     B200 hot path (SURVEY.md section 2): say so the way the reference reports fatal configuration
     problems -- log an error and exit -- instead of a traceback."""
-    hint = ("set traj_cluster.backend.hierarchical_on_device: true, or algorithm: kmeans"
-            if algorithm == "hierarchical" else "set traj_cluster.algorithm: kmeans")
+    flag = {"hierarchical": "hierarchical_on_device", "hdbscan": "hdbscan_on_device"}.get(algorithm)
+    hint = (f"set traj_cluster.backend.{flag}: true, or algorithm: kmeans" if flag
+            else "set traj_cluster.algorithm: kmeans")
     logger.error(f"Clustering algorithm '{algorithm}' is outside the B200 hot path; {hint}, "
                  "or use the reference package for it. Exiting...")
     sys.exit(1)

@@ -680,6 +680,80 @@ def linkage(Y: torch.Tensor, method: str = "complete", return_phases: bool = Fal
     return (Z, phases) if return_phases else Z
 
 
+# ---- N3: HDBSCAN core distances and mutual-reachability MST ---------------------------------------------
+def _hdbscan_frames(Y: torch.Tensor) -> torch.Tensor:
+    """The checks of ``linkage``: a CUDA (frames x features) tensor of at least 2 finite frames, returned
+    as contiguous float64 (float32 is widened exactly, as scikit-learn does)."""
+    _need_cuda("Y", Y)
+    if Y.dtype not in (torch.float32, torch.float64):
+        raise TypeError(f"Y must be float32 or float64, got {Y.dtype}")
+    if Y.dim() != 2 or Y.shape[0] < 2 or Y.shape[1] < 1:
+        raise ValueError("Y must be (frames x features) with at least 2 frames")
+    Y = Y.to(torch.float64).contiguous()
+    if not bool(torch.isfinite(Y).all()):
+        raise ValueError("Input contains NaN or infinity")
+    return Y
+
+
+def _hdbscan_workspace(dev, n: int, d: int, min_samples: int, extra: int, what: str) -> int:
+    """Workspace bytes of the HDBSCAN entry points, after checking that they and ``extra`` output bytes fit
+    in the free device memory."""
+    nbytes = int(_lib.load().dcg_hdbscan_workspace_bytes(n, d, min_samples))
+    if nbytes == 0:
+        raise ValueError(f"{n} frames are too many for HDBSCAN")
+    free, _ = torch.cuda.mem_get_info(dev)
+    if nbytes + extra > free:
+        raise MemoryError(f"{what} of {n} frames needs {nbytes + extra} bytes of device memory; {free} bytes are free")
+    return nbytes
+
+
+def core_distances(Y: torch.Tensor, min_samples: int) -> torch.Tensor:
+    """HDBSCAN core distances of the frames ``Y`` (n x d CUDA tensor, float32 or float64): the FP64
+    distance of every frame to its ``min_samples``-th nearest frame, the frame itself counted at distance
+    0.  Bitwise ``NearestNeighbors(n_neighbors=min_samples).kneighbors(X)[0][:, -1]`` (see dcg.h);
+    1 <= min_samples <= min(n, 64)."""
+    Y = _hdbscan_frames(Y)
+    n, d = Y.shape
+    min_samples = int(min_samples)
+    if min_samples > n:
+        # the wording of scikit-learn's kneighbors / HDBSCAN.fit check
+        raise ValueError(f"Expected n_neighbors <= n_samples_fit, but n_neighbors = {min_samples}, "
+                         f"n_samples_fit = {n}, n_samples = {n}")
+    if not 1 <= min_samples <= _lib.HDBSCAN_MAX_MIN_SAMPLES:
+        raise ValueError(f"min_samples must be in [1, {_lib.HDBSCAN_MAX_MIN_SAMPLES}], got {min_samples}")
+    _hdbscan_workspace(Y.device, n, d, min_samples, 8 * n, "core distances")
+    dev = Y.device
+    core = torch.empty(n, dtype=torch.float64, device=dev)
+    _call(dev, "dcg_core_distances_f64", Y.data_ptr(), n, d, d, min_samples, core.data_ptr(), None, 0, _stream(dev))
+    _count(1)
+    return core
+
+
+def mreach_mst(Y: torch.Tensor, core: torch.Tensor) -> torch.Tensor:
+    """Minimum spanning tree of the HDBSCAN mutual-reachability graph max(core_i, core_j, |y_i - y_j|):
+    the (n-1) x 3 FP64 rows (source node, new node, distance) in Prim's visiting order from frame 0,
+    bitwise sklearn's ``mst_from_data_matrix`` (sklearn/cluster/_hdbscan/_linkage.pyx; see dcg.h)."""
+    Y = _hdbscan_frames(Y)
+    n, d = Y.shape
+    _need_cuda("core", core, torch.float64)
+    if core.shape != (n,):
+        raise ValueError(f"core must have shape ({n},), got {tuple(core.shape)}")
+    core = core.contiguous()
+    if not bool(torch.isfinite(core).all()):
+        raise ValueError("core contains NaN or infinity")
+    nbytes = _hdbscan_workspace(Y.device, n, d, 1, 24 * (n - 1), "the mutual-reachability MST")
+    dev = Y.device
+    ws = _ws(nbytes, dev)
+    mst = torch.empty((n - 1, 3), dtype=torch.float64, device=dev)
+    _call(dev, "dcg_mreach_mst_f64", Y.data_ptr(), n, d, d, core.data_ptr(), mst.data_ptr(), ws.data_ptr(),
+          ws.numel(), _stream(dev))
+    _count(1)
+    steps = int(ws[:16].view(torch.int64)[1].item())
+    if steps != n - 1:
+        raise RuntimeError(f"mutual-reachability MST of {n} frames stopped after {steps} steps")
+    return mst
+
+
 # ---- E1: F x F generalised eigenproblem (leading eigenpairs) ---------------------------------------
 def tri_inv_blocks_(L: torch.Tensor, out: torch.Tensor, nblk: int, bs: int) -> torch.Tensor:
     """Inverses of the ``nblk`` diagonal blocks (``bs`` x ``bs``, at most 128) of the lower-triangular matrices

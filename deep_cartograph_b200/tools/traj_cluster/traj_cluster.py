@@ -1,11 +1,13 @@
-"""traj_cluster step API on the B200 backend (KMeans; agglomerative with ``backend.hierarchical_on_device``).
+"""traj_cluster step API on the B200 backend (KMeans; agglomerative with ``backend.hierarchical_on_device``;
+HDBSCAN with ``backend.hdbscan_on_device``).
 
 Same signature, return value and CSV layout as the reference's
 ``tools/traj_cluster/traj_cluster.py:18-113`` / ``traj_cluster_workflow.py:240-387``.
 Structure extraction (PDB / XTC), plots and the supplementary nearest-neighbour assignment are
 outside the hot path (SURVEY.md section 2).  ``algorithm: kmeans`` is accelerated, and so is
 ``algorithm: hierarchical`` (any of sklearn's four linkages, same tree and labels as sklearn) when the
-configuration sets ``backend: {hierarchical_on_device: true}``; HDBSCAN is not.
+configuration sets ``backend: {hierarchical_on_device: true}``, and ``algorithm: hdbscan`` (sklearn's
+labels, -1 for noise, in O(N) device memory) when it sets ``backend: {hdbscan_on_device: true}``.
 """
 from __future__ import annotations
 
@@ -62,8 +64,11 @@ class TrajClusterWorkflow:
             labels, centroids = statistics.cluster_data(X, self.configuration, self.initial_centroids)
         else:
             labels, centroids = statistics.optimize_clustering(X, self.configuration)
-        cv_data["cluster"] = labels
-        cv_data = statistics.find_centroids(cv_data, centroids, cv_labels)
+        cv_data["cluster"] = labels                        # -1: HDBSCAN noise
+        if len(centroids) == 0:                             # HDBSCAN found only noise: no frame is a centroid
+            cv_data["centroid"] = False
+        else:
+            cv_data = statistics.find_centroids(cv_data, centroids, cv_labels)
         frames = []
         for traj_index in range(len(self.cv_traj_paths)):
             n_samples = int((cv_data["traj_label"] == traj_index).sum())

@@ -1,8 +1,10 @@
 """Configuration contract of the traj_cluster step (reference ``yaml_schemas/traj_cluster.py:18-47``).
 
-The reference default algorithm is ``hierarchical``.  This backend accelerates ``kmeans`` and, when
+The reference default algorithm is ``hierarchical``.  This backend accelerates ``kmeans``; when
 ``backend.hierarchical_on_device`` is true, ``hierarchical`` (the same tree as scikit-learn, built on the
-device); otherwise ``hierarchical`` and ``hdbscan`` log an error and exit (SURVEY.md section 2).
+device); and when ``backend.hdbscan_on_device`` is true, ``hdbscan`` (the same labels as scikit-learn's
+HDBSCAN, in O(N) device memory).  Otherwise ``hierarchical`` and ``hdbscan`` log an error and exit
+(SURVEY.md section 2).
 Backend knobs live in the optional ``backend`` block."""
 from typing import Dict, List, Literal, Optional, Union
 
@@ -15,6 +17,9 @@ class Backend(BaseModel):
     # algorithm: hierarchical builds its tree on the device (bitwise the tree scikit-learn builds);
     # off by default, so a reference configuration keeps its current behaviour
     hierarchical_on_device: bool = False
+    # algorithm: hdbscan builds its single-linkage tree on the device (label for label scikit-learn's
+    # HDBSCAN); off by default for the same reason
+    hdbscan_on_device: bool = False
 
 
 class TrajClusterSchema(BaseModel):

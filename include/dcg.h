@@ -329,6 +329,28 @@ size_t dcg_linkage_workspace_bytes(int64_t n, int d, int method);
 int dcg_linkage_f64(const double* Y, int64_t n, int d, int64_t ld, int method, double* Z,
                     void* ws, size_t ws_bytes, void* stream);
 
+/* ---- N3: HDBSCAN single-linkage tree (core distances + mutual-reachability MST) -----------------------
+ * Replaces the device-side half of sklearn.cluster.HDBSCAN(metric="euclidean").fit on dense finite data,
+ * i.e. _hdbscan_prims (sklearn/cluster/_hdbscan/hdbscan.py) with its KD-tree.  O(n) memory, no n x n matrix.
+ * Distances are sqrt(sum_f (y_i[f] - y_j[f])^2), features ascending, a rounded multiply and a rounded add
+ * per term: the arithmetic of the KD-tree's and of EuclideanDistance.dist, so both results are bitwise
+ * sklearn's.
+ * dcg_core_distances_f64 replaces NearestNeighbors(n_neighbors=min_samples).kneighbors(X)[0][:, -1]:
+ *   core (n FP64) = distance of every frame to its min_samples-th nearest frame, the frame itself counted
+ *   at distance 0.  1 <= min_samples <= min(n, DCG_HDBSCAN_MAX_MIN_SAMPLES).  ws may be NULL.
+ * dcg_mreach_mst_f64 replaces sklearn/cluster/_hdbscan/_linkage.pyx mst_from_data_matrix (alpha = 1):
+ *   Prim from frame 0 on max(core[c], core[j], dist(c, j)); mst is (n-1) x 3 FP64 rows
+ *   (source node, new node, distance) in visiting order, the source being the tree node that last strictly
+ *   improved the new node.  The first 16 bytes of ws receive two int64 step counters.
+ * The edge sort (numpy's default argsort) and make_single_linkage are left to the caller.
+ * Errors: DCG_E_SHAPE for n < 2, d < 1, ld < d or min_samples out of range; DCG_E_NULL; DCG_E_WORKSPACE. */
+#define DCG_HDBSCAN_MAX_MIN_SAMPLES 64
+size_t dcg_hdbscan_workspace_bytes(int64_t n, int d, int min_samples);
+int dcg_core_distances_f64(const double* Y, int64_t n, int d, int64_t ld, int min_samples, double* core,
+                           void* ws, size_t ws_bytes, void* stream);
+int dcg_mreach_mst_f64(const double* Y, int64_t n, int d, int64_t ld, const double* core, double* mst,
+                       void* ws, size_t ws_bytes, void* stream);
+
 /* ---- N4: free-energy surface by binned kernel density estimation ---------------------------------
  * Replaces mlcolvar.utils.fes.compute_fes(backend="KDEpy") as called at modules/figures/figures.py:95
  * (from tools/train_colvars/train_colvars_workflow.py:146-182).  KDEpy's FFTKDE = linear binning onto
