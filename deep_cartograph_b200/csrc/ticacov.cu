@@ -11,66 +11,96 @@ namespace dcg {
 // A CTA stages kTcRowsPerCta rows (f row, g row, w, wl) in shared memory; thread e < d*d owns the
 // matrix entry (i, j) = (e / d, e % d) of BOTH matrices, thread d*d + i the three vector entries of
 // component i, thread d*d + d the two weight sums -- uniform code inside each class, rows unrolled
-// by 4, FP32 within the CTA's rows, FP64 across CTAs (one atomic per entry and CTA).
+// by 4, FP64 throughout.  The sums are raw, not mean-free, and the mean of the network outputs is
+// free to drift (the loss does not depend on it): C0 = sff/sw - mu mu^T then cancels |mu|^2 / var
+// digits, which FP32 partial sums (2^-24 of |mu|^2 per add) do not have to spare.  w * f_i of two
+// floats is exact in FP64, so each row costs one rounding per entry.
+// The result is deterministic: CTA k takes tiles k, k + G, k + 2G, ... (G = min(tiles, kTcMaxCtas))
+// and adds them in that order into its own column part[entry][k]; ticacov_reduce_kernel then sums
+// the G columns of each entry in a fixed order.  (FP64 atomics across CTAs would round differently
+// from run to run, since FP64 partial sums, unlike FP32 ones, do not add exactly.)
 constexpr int kTcThreads = 256;
 constexpr int kTcRowsPerCta = 128;
+constexpr int64_t kTcMaxCtas = 1024;
+
+static inline int64_t ticacov_ctas(int64_t B) { return min(ceil_div(B, kTcRowsPerCta), kTcMaxCtas); }
 
 __global__ void __launch_bounds__(kTcThreads)
 ticacov_kernel(const float* __restrict__ f, const float* __restrict__ g, const float* __restrict__ w,
-               const float* __restrict__ wl, int64_t B, int d, double* __restrict__ out) {
+               const float* __restrict__ wl, int64_t B, int d, double* __restrict__ part, int G) {
   extern __shared__ float sm[];              // [rows][2*d + 2] : f row, g row, w, wl
   const int stride = 2 * d + 2;
-  const int64_t r0 = (int64_t)blockIdx.x * kTcRowsPerCta;
-  const int rows = (int)min((int64_t)kTcRowsPerCta, B - r0);
-  for (int i = threadIdx.x; i < rows * d; i += kTcThreads) {
-    const int r = i / d, q = i - r * d;
-    sm[r * stride + q] = f[(r0 + r) * d + q];
-    sm[r * stride + d + q] = g[(r0 + r) * d + q];
-  }
-  for (int r = threadIdx.x; r < rows; r += kTcThreads) {
-    sm[r * stride + 2 * d] = w ? w[r0 + r] : 1.f;
-    sm[r * stride + 2 * d + 1] = wl ? wl[r0 + r] : 1.f;
-  }
-  __syncthreads();
   const int dd = d * d;
-  double* o_swf = out + 2;
-  double* o_sff = out + 2 + d;
-  double* o_sfg = o_sff + dd;
-  double* o_slf = o_sfg + dd;
-  double* o_slg = o_slf + d;
-  for (int e = threadIdx.x; e < dd + d + 1; e += kTcThreads) {
-    if (e < dd) {
-      const int i = e / d, j = e - i * d;
-      float a0 = 0.f, a1 = 0.f;
+  // part[idx][k]: this CTA's running sum of output entry idx
+  double* col = part + blockIdx.x;
+  const int64_t n_tiles = (B + kTcRowsPerCta - 1) / kTcRowsPerCta;
+  for (int64_t t = blockIdx.x; t < n_tiles; t += gridDim.x) {
+    const bool first = (t == (int64_t)blockIdx.x);
+    auto put = [&](int idx, double v) {
+      double* p = col + (size_t)idx * G;
+      *p = first ? v : *p + v;
+    };
+    const int64_t r0 = t * kTcRowsPerCta;
+    const int rows = (int)min((int64_t)kTcRowsPerCta, B - r0);
+    __syncthreads();                         // the previous tile's rows are no longer read
+    for (int i = threadIdx.x; i < rows * d; i += kTcThreads) {
+      const int r = i / d, q = i - r * d;
+      sm[r * stride + q] = f[(r0 + r) * d + q];
+      sm[r * stride + d + q] = g[(r0 + r) * d + q];
+    }
+    for (int r = threadIdx.x; r < rows; r += kTcThreads) {
+      sm[r * stride + 2 * d] = w ? w[r0 + r] : 1.f;
+      sm[r * stride + 2 * d + 1] = wl ? wl[r0 + r] : 1.f;
+    }
+    __syncthreads();
+    for (int e = threadIdx.x; e < dd + d + 1; e += kTcThreads) {
+      if (e < dd) {
+        const int i = e / d, j = e - i * d;
+        double a0 = 0.0, a1 = 0.0;
 #pragma unroll 4
-      for (int r = 0; r < rows; ++r) {
-        const float* row = sm + r * stride;
-        const float fi = row[i];
-        a0 = fmaf(row[2 * d] * fi, row[j], a0);
-        a1 = fmaf(row[2 * d + 1] * fi, row[d + j], a1);
-      }
-      atomicAdd(o_sff + e, (double)a0);
-      atomicAdd(o_sfg + e, (double)a1);
-    } else if (e < dd + d) {
-      const int i = e - dd;
-      float a0 = 0.f, a1 = 0.f, a2 = 0.f;
+        for (int r = 0; r < rows; ++r) {
+          const float* row = sm + r * stride;
+          const double fi = row[i];
+          a0 = fma((double)row[2 * d] * fi, (double)row[j], a0);
+          a1 = fma((double)row[2 * d + 1] * fi, (double)row[d + j], a1);
+        }
+        put(2 + d + e, a0);                  // sum w f f^T
+        put(2 + d + dd + e, a1);             // sum wl f g^T
+      } else if (e < dd + d) {
+        const int i = e - dd;
+        double a0 = 0.0, a1 = 0.0, a2 = 0.0;
 #pragma unroll 4
-      for (int r = 0; r < rows; ++r) {
-        const float* row = sm + r * stride;
-        a0 = fmaf(row[2 * d], row[i], a0);
-        a1 = fmaf(row[2 * d + 1], row[i], a1);
-        a2 = fmaf(row[2 * d + 1], row[d + i], a2);
+        for (int r = 0; r < rows; ++r) {
+          const float* row = sm + r * stride;
+          a0 = fma((double)row[2 * d], (double)row[i], a0);
+          a1 = fma((double)row[2 * d + 1], (double)row[i], a1);
+          a2 = fma((double)row[2 * d + 1], (double)row[d + i], a2);
+        }
+        put(2 + i, a0);                      // sum w f
+        put(2 + d + 2 * dd + i, a1);         // sum wl f
+        put(2 + 2 * d + 2 * dd + i, a2);     // sum wl g
+      } else {
+        double a0 = 0.0, a1 = 0.0;
+        for (int r = 0; r < rows; ++r) { a0 += sm[r * stride + 2 * d]; a1 += sm[r * stride + 2 * d + 1]; }
+        put(0, a0);
+        put(1, a1);
       }
-      atomicAdd(o_swf + i, (double)a0);
-      atomicAdd(o_slf + i, (double)a1);
-      atomicAdd(o_slg + i, (double)a2);
-    } else {
-      float a0 = 0.f, a1 = 0.f;
-      for (int r = 0; r < rows; ++r) { a0 += sm[r * stride + 2 * d]; a1 += sm[r * stride + 2 * d + 1]; }
-      atomicAdd(out + 0, (double)a0);
-      atomicAdd(out + 1, (double)a1);
     }
   }
+}
+
+// out[e] = sum over k of part[e][k], one warp per entry, in a fixed order (strided lane sums, then the
+// butterfly of warp_sum)
+__global__ void __launch_bounds__(kTcThreads)
+ticacov_reduce_kernel(const double* __restrict__ part, int G, int n_out, double* __restrict__ out) {
+  const int e = blockIdx.x * (kTcThreads / 32) + threadIdx.x / 32;
+  const int lane = threadIdx.x & 31;
+  if (e >= n_out) return;                    // warp-uniform
+  const double* p = part + (size_t)e * G;
+  double s = 0.0;
+  for (int k = lane; k < G; k += 32) s += p[k];
+  s = warp_sum(s);
+  if (lane == 0) out[e] = s;
 }
 
 // ---- A11: the d x d eigen-loss and its gradient in ONE launch ------------------------------------
@@ -83,8 +113,9 @@ ticacov_kernel(const float* __restrict__ f, const float* __restrict__ g, const f
 //  => dLoss/dC_tau = -2 sum lambda_i v_i v_i^T,   dLoss/dC0 = +2 sum lambda_i^2 v_i v_i^T.
 // In torch this is ~40 tiny launches (cholesky, two triangular solves, eigvalsh and their
 // backward); here one warp does it in shared memory (d <= 32).
-// res layout (doubles): [0] loss, [1] status (0 ok, 1 = B not positive definite), [2] sum w,
-// [3] sum wl, then evals[d] (descending), mu[d], G0[d*d], Gt[d*d].
+// res layout (doubles): [0] loss, [1] status (0 ok, 1 = B not positive definite or a sum not finite;
+// then loss and evals are NaN and G0 = Gt = 0), [2] sum w, [3] sum wl, then evals[d] (descending),
+// mu[d], G0[d*d], Gt[d*d].
 __global__ void __launch_bounds__(32)
 ticaloss_kernel(const double* __restrict__ sums, int d, double reg, int n_eig, double* __restrict__ res) {
   __shared__ double C0[32][33], Ct[32][33], L[32][33], A[32][33], V[32][33];
@@ -118,6 +149,12 @@ ticaloss_kernel(const double* __restrict__ sums, int d, double reg, int n_eig, d
       C0[i][j] = 0.5 * (L[i][j] + L[j][i]);
       Ct[i][j] = 0.5 * (A[i][j] + A[j][i]);
     }
+    // a NaN / Inf anywhere in the sums (a diverged network, sum w = 0 or sum wl = 0) reaches mu, nu, xi, C0
+    // or C_tau, except an infinite sum w / sum wl, which zeroes what it divides: flag all of it here, as the
+    // Cholesky below only sees C0's pivots
+    bool fin = isfinite(sw) && isfinite(swl) && isfinite(mu[i]) && isfinite(nu[i]) && isfinite(xi[i]);
+    for (int j = 0; j < d; ++j) fin = fin && isfinite(C0[i][j]) && isfinite(Ct[i][j]);
+    if (!fin) s_bad = 1;
   }
   __syncwarp();
   // Cholesky of B = C0 + reg I (column by column; lanes own rows)
@@ -217,13 +254,16 @@ ticaloss_kernel(const double* __restrict__ sums, int d, double reg, int n_eig, d
         }
       }
   }
-  // eigenvalues descending (rank by counting; ties broken by index)
+  // eigenvalues descending (rank by counting; ties broken by index).  A permutation only if every key
+  // compares, so NaN ranks as -inf, as in gen_eig_small_kernel: otherwise ranks collide and order[] keeps
+  // unwritten slots that index V below
   if (lane < d) {
     const double mine = A[lane][lane];
+    const double km = (mine == mine) ? mine : -INFINITY;
     int r = 0;
     for (int j = 0; j < d; ++j) {
-      const double o = A[j][j];
-      r += (o > mine) || (o == mine && j < lane);
+      const double o = (A[j][j] == A[j][j]) ? A[j][j] : -INFINITY;
+      r += (o > km) || (o == km && j < lane);
     }
     order[r] = lane;
     ev[r] = mine;
@@ -255,7 +295,7 @@ ticaloss_kernel(const double* __restrict__ sums, int d, double reg, int n_eig, d
   double* o_gt = o_g0 + dd;
   if (lane < d) {
     const int i = lane;
-    o_ev[i] = ev[i];
+    o_ev[i] = s_bad ? NAN : ev[i];
     o_mu[i] = mu[i];
     for (int j = 0; j < d; ++j) {
       double g0 = 0.0, gt = 0.0;
@@ -433,15 +473,25 @@ extern "C" size_t dcg_ticacov_out_doubles(int d) {
   return (size_t)(2 + d + 2 * d * d + 2 * d);
 }
 
+extern "C" size_t dcg_ticacov_workspace_bytes(int64_t B, int d) {
+  if (B <= 0 || d < 1 || d > 32) return 0;
+  return (size_t)ticacov_ctas(B) * dcg_ticacov_out_doubles(d) * sizeof(double);
+}
+
 extern "C" int dcg_ticacov_f32(const float* f, const float* g, const float* w, const float* wl,
-                               int64_t B, int d, double* out, void* stream) {
+                               int64_t B, int d, double* out, void* ws, size_t ws_bytes, void* stream) {
   if (!f || !g || !out) return DCG_E_NULL;
   if (B <= 0 || d < 1 || d > 32) return DCG_E_SHAPE;
+  if (!ws || ws_bytes < dcg_ticacov_workspace_bytes(B, d)) return DCG_E_WORKSPACE;
   cudaStream_t st = (cudaStream_t)stream;
-  DCG_CUDA_TRY(cudaMemsetAsync(out, 0, dcg_ticacov_out_doubles(d) * sizeof(double), st));
+  const int G = (int)ticacov_ctas(B);
+  const int n_out = (int)dcg_ticacov_out_doubles(d);
   const size_t smem = (size_t)kTcRowsPerCta * (2 * d + 2) * sizeof(float);
   DCG_CUDA_TRY(ensure_dynamic_smem((const void*)ticacov_kernel, (size_t)(smem)));
-  ticacov_kernel<<<(unsigned)ceil_div(B, kTcRowsPerCta), kTcThreads, smem, st>>>(f, g, w, wl, B, d, out);
+  ticacov_kernel<<<G, kTcThreads, smem, st>>>(f, g, w, wl, B, d, (double*)ws, G);
+  DCG_LAUNCH_CHECK();
+  ticacov_reduce_kernel<<<(unsigned)ceil_div(n_out, kTcThreads / 32), kTcThreads, 0, st>>>((const double*)ws, G,
+                                                                                          n_out, out);
   DCG_LAUNCH_CHECK();
   return 0;
 }

@@ -503,10 +503,17 @@ def nearest_to_centers(Y: torch.Tensor, centers: torch.Tensor) -> torch.Tensor:
 # ---- A11 --------------------------------------------------------------------------------------
 def ticacov_sums(f: torch.Tensor, g: torch.Tensor, w: Optional[torch.Tensor] = None,
                  wl: Optional[torch.Tensor] = None) -> dict:
-    """Weighted raw correlation sums of DeepTICA network outputs (B x d, float32)."""
+    """Weighted raw correlation sums of DeepTICA network outputs (B x d, float32).  ``g`` must
+    have the shape of ``f``, and ``w`` / ``wl`` (if given) B elements on the same device."""
+    # the kernel reads B rows of g and B weights: a shorter tensor would be read past its end
+    if f.dim() != 2 or g.shape != f.shape:
+        raise ValueError(f"f and g must be (B, d) of one shape, got {tuple(f.shape)} and {tuple(g.shape)}")
+    B, d = f.shape
+    for name, v in (("w", w), ("wl", wl)):
+        if v is not None and (v.dim() != 1 or v.numel() != B or v.device != f.device):
+            raise ValueError(f"{name} must be a ({B},) tensor on {f.device}, got {tuple(v.shape)} on {v.device}")
     _need_cuda("f", f, torch.float32)
     _need_cuda("g", g, torch.float32)
-    B, d = f.shape
     f = f.contiguous()
     g = g.contiguous()
     lib = _lib.load()
@@ -518,9 +525,10 @@ def ticacov_sums(f: torch.Tensor, g: torch.Tensor, w: Optional[torch.Tensor] = N
         w = w.to(torch.float32).contiguous()
     if wl is not None:
         wl = wl.to(torch.float32).contiguous()
+    ws = _ws(lib.dcg_ticacov_workspace_bytes(B, d), f.device)
     _call(f.device, "dcg_ticacov_f32", f.data_ptr(), g.data_ptr(), _ptr(w), _ptr(wl), B, d,
-              out.data_ptr(), _stream(f.device))
-    _count(1)
+              out.data_ptr(), ws.data_ptr(), ws.numel(), _stream(f.device))
+    _count(2)
     o = 2 + d
     return {"flat": out, "sw": out[0], "swl": out[1], "swf": out[2:o],
             "sff": out[o:o + d * d].view(d, d), "sfg": out[o + d * d:o + 2 * d * d].view(d, d),

@@ -241,14 +241,18 @@ int dcg_nearest_to_centers(const void* Y, int64_t n, int d, int64_t ld, int dtyp
 /* ---- A11: DeepTICA minibatch covariance ------------------------------------------------------
  * Replaces the correlation sums inside mlcolvar `DeepTICA.training_step` (driven from
  * cv_calculator.py:1508-1524).  f, g are B x d float32 network outputs (row-major), w / wl the
- * per-sample weights (NULL = 1).  Outputs FP64 raw sums (overwritten):
+ * per-sample weights (NULL = 1).  Outputs FP64 raw sums (overwritten), accumulated in FP64 from
+ * the first row (each w f_i f_j is rounded once), since they are not mean-free:
  *   out[0]            = sum w,          out[1] = sum wl
  *   out[2 .. 2+d)     = sum w f
  *   then d*d each     : sum w f f^T,  sum wl f g^T,  then d each: sum wl f, sum wl g
- * The caller forms mean-free C0 / C_tau in FP64 (see host code).  1 <= d <= 32.                 */
+ * The caller forms mean-free C0 / C_tau in FP64 (see host code).  1 <= d <= 32.  The result is
+ * deterministic: the per-CTA partial sums go to ws (dcg_ticacov_workspace_bytes(B, d) bytes, no
+ * initialisation needed) and are added in a fixed order by a second launch.                      */
 size_t dcg_ticacov_out_doubles(int d);
+size_t dcg_ticacov_workspace_bytes(int64_t B, int d);
 int dcg_ticacov_f32(const float* f, const float* g, const float* w, const float* wl,
-                    int64_t B, int d, double* out, void* stream);
+                    int64_t B, int d, double* out, void* ws, size_t ws_bytes, void* stream);
 
 /* ---- A11: DeepTICA eigen-loss and its gradient ------------------------------------------------
  * Replaces mlcolvar `cholesky_eigh` + `ReduceEigenvaluesLoss(mode='sum2')` and their autograd
@@ -257,8 +261,9 @@ int dcg_ticacov_f32(const float* f, const float* g, const float* w, const float*
  * mean-free symmetrised C0 / C_tau, B = C0 + reg I, L = chol(B), the eigenvalues of
  * L^-1 C_tau L^-T (descending) and loss = -sum_{i < n_eig} lambda_i^2 (n_eig <= 0: all), together
  * with dLoss/dC0 and dLoss/dC_tau (symmetric d x d).
- * res (doubles): [0] loss, [1] status (0 ok, 1: B not positive definite, loss = NaN), [2] sum w,
- * [3] sum wl, evals[d], mu[d] (weighted mean of f), G0[d*d], Gt[d*d].                            */
+ * res (doubles): [0] loss, [1] status (0 ok, 1: B not positive definite or a sum, mean or
+ * covariance not finite -- then loss and evals are NaN and G0 = Gt = 0), [2] sum w, [3] sum wl,
+ * evals[d], mu[d] (weighted mean of f), G0[d*d], Gt[d*d].                                        */
 size_t dcg_ticaloss_out_doubles(int d);
 int dcg_ticaloss_f64(const double* sums, int d, double reg, int n_eig, double* res, void* stream);
 
