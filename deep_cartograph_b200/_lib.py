@@ -82,6 +82,8 @@ _SIGNATURES = {
     "dcg_hdbscan_workspace_bytes": (_c_sz, [_c_i64, _c_int, _c_int]),
     "dcg_core_distances_f64": (_c_int, [_p, _c_i64, _c_int, _c_i64, _c_int, _p, _p, _c_sz, _p]),
     "dcg_mreach_mst_f64": (_c_int, [_p, _c_i64, _c_int, _c_i64, _p, _p, _p, _c_sz, _p]),
+    "dcg_nearest_frames_workspace_bytes": (_c_sz, [_c_i64, _c_i64, _c_int]),
+    "dcg_nearest_frames_f64": (_c_int, [_p, _c_i64, _c_i64, _p, _c_i64, _c_i64, _c_int, _p, _p, _p, _c_sz, _p]),
     "dcg_fes_bin_f32": (_c_int, [_p, _c_i64, _c_i64, _c_int, _c_int, C.c_double, C.c_double, C.c_double, C.c_double,
                                  _c_int, _c_int, _p, _p, _p]),
     "dcg_fes_smooth_f64": (_c_int, [_p, _c_int, _c_int, _c_int, C.c_double, C.c_double, C.c_double, _p, _p, _p, _p]),

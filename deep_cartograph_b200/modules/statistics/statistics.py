@@ -703,6 +703,23 @@ def hdbscan_clustering(feature_matrix, settings: Dict) -> Tuple[np.ndarray, np.n
     return labels, means
 
 
+def assign_closest_cluster(clustered, labels, sup) -> np.ndarray:
+    """Label of the nearest clustered frame of every supplementary frame (reference
+    ``traj_cluster_workflow.py:207-238``, ``assign_closest_cluster``).  The reference's semantics are assumed
+    to be ``NearestNeighbors(n_neighbors=1).fit(clustered).kneighbors(sup)``, each supplementary frame taking
+    the label of the returned frame; the search runs on the device (``ops.nearest_frames``) with the KD-tree's
+    distance arithmetic, and among exactly tied nearest frames the lowest-indexed one wins (scikit-learn's
+    KD-tree returns whichever tied frame it visits first).  HDBSCAN noise (-1) propagates: a frame whose
+    nearest clustered frame is noise is noise."""
+    labels = np.asarray(labels)
+    X = _to_device(clustered)
+    if labels.shape != (X.shape[0],):
+        raise ValueError(f"labels must have one entry per clustered frame ({X.shape[0]}), got shape {labels.shape}")
+    Q = _to_device(sup)
+    index, _ = ops.nearest_frames(X, Q)
+    return labels[index.cpu().numpy()]
+
+
 def _outside_hot_path(algorithm):
     """hierarchical clustering and hdbscan without their ``backend.*_on_device`` flag are not part of the
     B200 hot path (SURVEY.md section 2): say so the way the reference reports fatal configuration

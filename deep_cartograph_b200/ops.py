@@ -762,6 +762,63 @@ def mreach_mst(Y: torch.Tensor, core: torch.Tensor) -> torch.Tensor:
     return mst
 
 
+# ---- N5: nearest clustered frame of supplementary frames -------------------------------------------------
+NEAREST_QUERY_BLOCK = 128          # queries of one CTA of the search kernel (kQB, csrc/nearest.cu)
+
+
+def _nearest_rows(name: str, Y: torch.Tensor) -> torch.Tensor:
+    _need_cuda(name, Y)
+    if Y.dtype not in (torch.float32, torch.float64):
+        raise TypeError(f"{name} must be float32 or float64, got {Y.dtype}")
+    if Y.dim() != 2 or Y.shape[1] < 1:
+        raise ValueError(f"{name} must be (frames x features) with at least 1 feature")
+    Y = Y.to(torch.float64).contiguous()
+    if not bool(torch.isfinite(Y).all()):
+        raise ValueError(f"{name} contains NaN or infinity")
+    return Y
+
+
+def nearest_frames(X: torch.Tensor, Q: torch.Tensor, return_counters: bool = False):
+    """For every query frame of ``Q`` (m x d) its nearest frame of ``X`` (n x d): ``(index int64, dist float64)``.
+    CUDA tensors, float32 (widened exactly) or float64, finite, n >= 1.  dist is the FP64 Euclidean distance
+    with scikit-learn's KD-tree arithmetic, so it is bitwise ``NearestNeighbors(n_neighbors=1,
+    algorithm="kd_tree").fit(X).kneighbors(Q)``'s; among frames at exactly the same distance the lowest index
+    is returned (see dcg.h, N5).  ``return_counters``: also return (tiles visited, tiles considered)."""
+    X = _nearest_rows("X", X)
+    Q = _nearest_rows("Q", Q)
+    if X.shape[0] < 1:
+        raise ValueError("X must hold at least 1 frame")
+    if Q.shape[1] != X.shape[1]:
+        raise ValueError(f"X and Q must have the same number of features, got {X.shape[1]} and {Q.shape[1]}")
+    if X.device != Q.device:
+        raise ValueError(f"X and Q must be on the same device, got {X.device} and {Q.device}")
+    n, d = X.shape
+    m = Q.shape[0]
+    dev = X.device
+    if m == 0:
+        index, dist = torch.empty(0, dtype=torch.int64, device=dev), torch.empty(0, dtype=torch.float64, device=dev)
+        return (index, dist, (0, 0)) if return_counters else (index, dist)
+    with torch.cuda.device(dev):
+        nbytes = int(_lib.load().dcg_nearest_frames_workspace_bytes(n, m, d))
+    if nbytes == 0:
+        raise ValueError(f"nearest frames of {m} queries among {n} frames of {d} features: shape out of range")
+    free, _ = torch.cuda.mem_get_info(dev)
+    if nbytes + 16 * m > free:
+        raise MemoryError(f"nearest frames of {m} queries among {n} frames needs {nbytes + 16 * m} bytes of device "
+                          f"memory; {free} bytes are free")
+    ws = _ws(nbytes, dev)
+    index = torch.empty(m, dtype=torch.int64, device=dev)
+    dist = torch.empty(m, dtype=torch.float64, device=dev)
+    _call(dev, "dcg_nearest_frames_f64", X.data_ptr(), n, d, Q.data_ptr(), m, d, d, index.data_ptr(),
+          dist.data_ptr(), ws.data_ptr(), ws.numel(), _stream(dev))
+    _count(8)                      # box, keys, ordered copies, tile boxes, search; plus two radix sorts
+    visited, considered = (int(v) for v in ws[:16].view(torch.int64).tolist())
+    blocks = -(-m // NEAREST_QUERY_BLOCK)
+    if not (blocks <= visited <= considered and considered % blocks == 0):
+        raise ValueError(f"nearest-frame search visited {visited} of {considered} tiles for {blocks} query blocks")
+    return (index, dist, (visited, considered)) if return_counters else (index, dist)
+
+
 # ---- E1: F x F generalised eigenproblem (leading eigenpairs) ---------------------------------------
 def tri_inv_blocks_(L: torch.Tensor, out: torch.Tensor, nblk: int, bs: int) -> torch.Tensor:
     """Inverses of the ``nblk`` diagonal blocks (``bs`` x ``bs``, at most 128) of the lower-triangular matrices

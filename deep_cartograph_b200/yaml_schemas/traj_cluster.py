@@ -4,7 +4,8 @@ The reference default algorithm is ``hierarchical``.  This backend accelerates `
 ``backend.hierarchical_on_device`` is true, ``hierarchical`` (the same tree as scikit-learn, built on the
 device); and when ``backend.hdbscan_on_device`` is true, ``hdbscan`` (the same labels as scikit-learn's
 HDBSCAN, in O(N) device memory).  Otherwise ``hierarchical`` and ``hdbscan`` log an error and exit
-(SURVEY.md section 2).
+(SURVEY.md section 2).  Supplementary trajectories need no setting: when the step is given
+``sup_cv_traj_paths``, their frames take the cluster of their nearest clustered frame, on the device.
 Backend knobs live in the optional ``backend`` block."""
 from typing import Dict, List, Literal, Optional, Union
 

@@ -356,6 +356,27 @@ int dcg_core_distances_f64(const double* Y, int64_t n, int d, int64_t ld, int mi
 int dcg_mreach_mst_f64(const double* Y, int64_t n, int d, int64_t ld, const double* core, double* mst,
                        void* ws, size_t ws_bytes, void* stream);
 
+/* ---- N5: nearest clustered frame of supplementary frames ----------------------------------------------
+ * Replaces the NearestNeighbors(n_neighbors=1).fit(X).kneighbors(Q) of the reference's assign_closest_cluster
+ * (tools/traj_cluster/traj_cluster_workflow.py:207-238): for each of the m queries Q (row stride ldq) the
+ * nearest of the n frames X (row stride ldx), all d features, FP64 (csrc/nearest.cu).
+ * rdist = sum_f (q_f - x_f)^2, features ascending, a rounded subtract, multiply and add per term, then one
+ * sqrt: the arithmetic of scikit-learn's KD-tree, which its `auto` algorithm picks for d <= 15; the device
+ * keeps it for every d (for d > 15 scikit-learn switches to brute force with the GEMM expansion).
+ * index[i] (int64) = the lexicographic minimum of (rdist, frame index), i.e. the lowest-indexed frame among
+ * exact ties; dist[i] = sqrt(rdist).  The frames are put in Morton order and cut into tiles whose boxes
+ * prune the search exactly (the bound uses the same rounded arithmetic; see nearest.cu).  Memory is
+ * O((n + m) d), no n x m buffer.  The first 16 bytes of ws receive two uint64 counters: tiles visited and
+ * tiles considered (query blocks x tiles).  The workspace query needs a CUDA device (it sizes the radix
+ * sort) and returns 0 without one or for an invalid shape.  m = 0 is a no-op.  Every coordinate of X and Q
+ * must be finite (ops.nearest_frames checks it): with NaN in a query's row no frame compares below its best, and
+ * its index and dist are then not defined.
+ * Errors: DCG_E_SHAPE for n < 1, m < 0, d < 1, d > 8192, ldx < d, ldq < d or n or m above INT_MAX;
+ * DCG_E_NULL; DCG_E_WORKSPACE.                                                                         */
+size_t dcg_nearest_frames_workspace_bytes(int64_t n, int64_t m, int d);
+int dcg_nearest_frames_f64(const double* X, int64_t n, int64_t ldx, const double* Q, int64_t m, int64_t ldq,
+                           int d, int64_t* index, double* dist, void* ws, size_t ws_bytes, void* stream);
+
 /* ---- N4: free-energy surface by binned kernel density estimation ---------------------------------
  * Replaces mlcolvar.utils.fes.compute_fes(backend="KDEpy") as called at modules/figures/figures.py:95
  * (from tools/train_colvars/train_colvars_workflow.py:146-182).  KDEpy's FFTKDE = linear binning onto
