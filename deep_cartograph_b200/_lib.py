@@ -71,11 +71,6 @@ _SIGNATURES = {
     "dcg_ticacov_f32": (_c_int, [_p, _p, _p, _p, _c_i64, _c_int, _p, _p, _c_sz, _p]),
     "dcg_gen_eig_small_f64": (_c_int, [_p, _p, _c_int, _c_int, _p, _p, _p, _p]),
     "dcg_tri_inv_blocks_f64": (_c_int, [_p, _p, _c_int, _c_int, _c_int, _c_i64, _c_i64, _c_i64, _c_i64, _c_i64, _c_i64, _p]),
-    "dcg_eig_shift_matrix_f64": (_c_int, [_p, _p, _c_int, C.c_double, _p, _p, _p]),
-    "dcg_eig_chol_inv_workspace_bytes": (_c_sz, [_c_int]),
-    "dcg_eig_chol_inv_f64": (_c_int, [_p, _c_int, _p, _p, _p, _p, _c_sz, _p]),
-    "dcg_eig_iterate_workspace_bytes": (_c_sz, [_c_int, _c_int, _c_int]),
-    "dcg_eig_iterate_f64": (_c_int, [_p, _p, _p, _p, _p, _c_int, _c_int, _c_int, _c_int, _p, _p, _p, _p, _p, _p, _c_sz, _p]),
     "dcg_cluster_dispersion": (_c_int, [_p, _c_i64, _c_int, _c_i64, _c_int, _p, _p, _c_int, _p, _p, _p]),
     "dcg_linkage_workspace_bytes": (_c_sz, [_c_i64, _c_int, _c_int]),
     "dcg_linkage_f64": (_c_int, [_p, _c_i64, _c_int, _c_i64, _c_int, _p, _p, _c_sz, _p]),

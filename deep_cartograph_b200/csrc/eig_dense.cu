@@ -1,619 +1,6 @@
-// E1: the F x F generalised eigenproblem of TICA on one device, hand-written FP64.
-// Replaces mlcolvar `cholesky_eigh` inside `TICA.compute` as called at reference cv_calculator.py:2257-2261
-// (and :2350-2354, :2374-2378 for hTICA) for the LEADING eigenpairs, which is all the reference keeps.
-//
-// Shift-and-invert subspace iteration on the pencil (Ct, B), B = C0 + reg I (linalg.py has the maths):
-//     K = sigma B - Ct  (SPD for sigma > lambda_max);   X <- K^-1 B X   + Rayleigh-Ritz.
-// The F x F work is FP64 products of an F x F matrix with an F x b block (b = d + 8 <= 32) -- ~50 of
-// them per solve, each a few microseconds of work, which as separate library GEMMs cost 9 us apiece
-// plus launch gaps (round 1: 2.65 ms at F = 1000, 1.9 ms of it GPU time, the rest gaps) -- and one
-// Cholesky factorisation with its triangular inverse.  Here they are two persistent cooperative kernels
-// (one CTA per SM, grid barriers on a global counter):
-//
-//   eig_iterate_kernel   all iterations of  Z = B X;  Y = Li^T (Li Z);  R = Z - K Y;  Y += Li^T (Li R);  X = Y
-//                        (explicit inverse factor Li = chol(K)^-1 + one step of iterative refinement),
-//                        lazy column normalisation, one Cholesky-QR re-orthogonalisation, then the
-//                        Rayleigh-Ritz products BX = B X, CX = Ct X, Gb = X^T BX, H = X^T CX.
-//                        A product assigns one warp per matrix row; the F x b block is staged transposed
-//                        in shared memory (conflict-free, read through L2: other CTAs just wrote it).
-//   eig_chol_inv_kernel  blocked right-looking Cholesky (32 x 32 diagonal blocks factored and inverted by
-//                        one warp in registers, with shuffles; the next diagonal block is prepared inside
-//                        the trailing update, two grid barriers per block step) and the triangular inverse
-//                        by independent block columns.
-// Roofline: neither HBM nor tensor -- latency of ~60 dependent steps; reported in seconds (SURVEY 8d).
-#include <cstdlib>
+// Eigen stage of TICA (linalg.py): inverses of the diagonal blocks of chol(K) for its explicit inverse.
+// The rest of the shift-and-invert iteration is cuSOLVER / cuBLAS calls and dcg_gen_eig_small_f64 (ticacov.cu).
 #include "dcg_common.cuh"
-
-namespace dcg {
-namespace {
-
-constexpr int kEigThreads = 256;
-constexpr int kEigWarps = kEigThreads / 32;
-constexpr int kMaxB = 32;
-
-__device__ __forceinline__ unsigned ld_acquire_u32(const unsigned* p) {
-  unsigned v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-
-// All CTAs of the (cooperatively launched, hence co-resident) grid meet here.  `epoch` counts the
-// barriers this CTA has passed; the counter only grows.  counter[1] is an abort flag: a CTA that has
-// spun for ~1 s gives up, raises it, and every later barrier falls through (the caller sees it in the
-// status word) -- a lost CTA must not hang the device.
-__device__ __forceinline__ void grid_barrier(unsigned* counter, unsigned& epoch) {
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    __threadfence();
-    const unsigned target = (++epoch) * gridDim.x;
-    atomicAdd(counter, 1u);
-    unsigned spins = 0;
-    while (ld_acquire_u32(counter) < target) {
-      if ((++spins & 0xFFFu) == 0) {
-        if (ld_acquire_u32(counter + 1) != 0u) break;
-        if (spins > (1u << 21)) {                       // ~1 s of polling
-          counter[2] = epoch; counter[3] = ld_acquire_u32(counter); counter[4] = blockIdx.x;
-          atomicExch(counter + 1, 1u);
-          break;
-        }
-      }
-    }
-    __threadfence();
-  }
-  __syncthreads();
-}
-
-__device__ __forceinline__ double shfl_d(double v, int src) { return __shfl_sync(0xffffffffu, v, src); }
-
-struct IterParams {
-  const double* B;
-  const double* K;
-  const double* Ct;
-  const double* Li;      // chol(K)^-1, lower triangular, row-major
-  const double* LiT;     // its transpose
-  double* X;             // F x b, row-major (in: start block, out: iterated block, columns normalised)
-  double* Z; double* T; double* Y; double* R;     // F x b scratch
-  double* BX; double* CX;                          // F x b outputs
-  double* small;         // [colsq: (n_iter + 1) x 32 | G: 32 x 32 | Gb: 32 x 32 | H: 32 x 32], zeroed by the host
-  unsigned* barrier;     // zeroed by the host
-  int F, b, n_iter, cholqr_at, kc;
-};
-
-enum { kFull = 0, kLower = 1, kUpper = 2 };
-
-// U[r][j] = sum_k A[r][k] V[k][j] * vscale[j] for the rows of this CTA's warps; epi(r, j, value) runs on
-// lane j < b.  One warp per row and pass; V is staged transposed in shared memory in chunks of kc rows.
-template <class Epi>
-__device__ __forceinline__ void block_product(const double* __restrict__ A, int F, int tri, const double* V,
-                                              const double* vscale, int b, int kc, double* sV, Epi epi) {
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int rows_per_pass = gridDim.x * kEigWarps;
-  for (int r0 = 0; r0 < F; r0 += rows_per_pass) {
-    const int r = r0 + blockIdx.x * kEigWarps + warp;
-    double acc[kMaxB];
-#pragma unroll
-    for (int j = 0; j < kMaxB; ++j) acc[j] = 0.0;
-    for (int k0 = 0; k0 < F; k0 += kc) {
-      const int kn = min(kc, F - k0);
-      __syncthreads();
-      {
-        // stage V[k0 .. k0+kn) transposed; 8 independent L2 loads in flight per thread
-        const int total = kn * b;
-        const double* src = V + (size_t)k0 * b;
-        for (int base = threadIdx.x; base < total; base += kEigThreads * 8) {
-          double v[8];
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            const int i = base + u * kEigThreads;
-            v[u] = i < total ? __ldcg(src + i) : 0.0;          // written by other CTAs: read through L2
-          }
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            const int i = base + u * kEigThreads;
-            if (i < total) {
-              const int k = i / b, j = i - k * b;
-              sV[j * kc + k] = vscale ? v[u] * vscale[j] : v[u];
-            }
-          }
-        }
-      }
-      __syncthreads();
-      if (r < F) {
-        int lo = k0, hi = k0 + kn;
-        if (tri == kLower) hi = min(hi, r + 1);
-        if (tri == kUpper) lo = max(lo, r);
-        const double* arow = A + (size_t)r * F;
-        for (int k = lo + lane; k < hi; k += 32 * 8) {
-          double a[8];
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            const int kk = k + 32 * u;
-            a[u] = kk < hi ? __ldg(arow + kk) : 0.0;
-          }
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            const int kk = min(k + 32 * u, hi - 1);            // a[u] is 0 beyond hi; keep the address in range
-            const double* sv = sV + (kk - k0);
-#pragma unroll
-            for (int j = 0; j < kMaxB; ++j)
-              if (j < b) acc[j] = fma(a[u], sv[j * kc], acc[j]);
-          }
-        }
-      }
-    }
-    double mine = 0.0;
-#pragma unroll
-    for (int j = 0; j < kMaxB; ++j) {
-      if (j < b) {
-        double v = acc[j];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-        if (lane == j) mine = v;
-      }
-    }
-    if (r < F && lane < b) epi(r, lane, mine);
-  }
-}
-
-// G[i][j] += sum over this CTA's rows of P[r][i] * Q[r][j]  (P, Q: F x b, rows of this CTA's warps),
-// reduced through shared memory, then one global atomic per CTA and entry.
-__device__ __forceinline__ void gram_accumulate(const double* P, const double* Q, int F, int b, double* sG, double* G) {
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  for (int i = threadIdx.x; i < b * b; i += kEigThreads) sG[i] = 0.0;
-  __syncthreads();
-  const int rows_per_pass = gridDim.x * kEigWarps;
-  for (int r0 = 0; r0 < F; r0 += rows_per_pass) {
-    const int r = r0 + blockIdx.x * kEigWarps + warp;
-    if (r >= F) continue;
-    const double p = lane < b ? __ldcg(P + (size_t)r * b + lane) : 0.0;
-    const double q = lane < b ? __ldcg(Q + (size_t)r * b + lane) : 0.0;
-    for (int i = 0; i < b; ++i) {
-      const double pi = shfl_d(p, i);
-      if (lane < b) atomicAdd(&sG[i * b + lane], pi * q);
-    }
-  }
-  __syncthreads();
-  for (int i = threadIdx.x; i < b * b; i += kEigThreads) atomicAdd(&G[i], sG[i]);
-}
-
-__global__ void __launch_bounds__(kEigThreads, 1) eig_iterate_kernel(const IterParams p) {
-  extern __shared__ __align__(16) double smem_d[];
-  double* sV = smem_d;                                  // b x kc
-  __shared__ double sS[kMaxB];                          // column scales
-  __shared__ double sG[kMaxB * kMaxB], sL[kMaxB * kMaxB];
-  const int F = p.F, b = p.b, kc = p.kc;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  unsigned epoch = 0;
-  double* colsq = p.small;
-  double* G = p.small + (size_t)(p.n_iter + 1) * 32;
-  double* Gb = G + 1024;
-  double* H = Gb + 1024;
-  const int rows_per_pass = gridDim.x * kEigWarps;
-  bool scale_pending = false;                           // X carries un-applied column norms (slot it)
-  int scale_slot = 0;
-
-  for (int it = 0; it < p.n_iter; ++it) {
-    // column scales of X from the sums of squares accumulated when X was written
-    if (threadIdx.x < b) sS[threadIdx.x] = scale_pending ? rsqrt(__ldcg(colsq + scale_slot * 32 + threadIdx.x)) : 1.0;
-    __syncthreads();
-    // Z = B (X s)
-    block_product(p.B, F, kFull, p.X, sS, b, kc, sV, [&](int r, int j, double v) { p.Z[(size_t)r * b + j] = v; });
-    grid_barrier(p.barrier, epoch);
-    // T = Li Z ; Y = Li^T T
-    block_product(p.Li, F, kLower, p.Z, nullptr, b, kc, sV, [&](int r, int j, double v) { p.T[(size_t)r * b + j] = v; });
-    grid_barrier(p.barrier, epoch);
-    block_product(p.LiT, F, kUpper, p.T, nullptr, b, kc, sV, [&](int r, int j, double v) { p.Y[(size_t)r * b + j] = v; });
-    grid_barrier(p.barrier, epoch);
-    // R = Z - K Y   (one step of iterative refinement of the explicit-inverse solve)
-    block_product(p.K, F, kFull, p.Y, nullptr, b, kc, sV,
-                  [&](int r, int j, double v) { p.R[(size_t)r * b + j] = __ldcg(p.Z + (size_t)r * b + j) - v; });
-    grid_barrier(p.barrier, epoch);
-    block_product(p.Li, F, kLower, p.R, nullptr, b, kc, sV, [&](int r, int j, double v) { p.T[(size_t)r * b + j] = v; });
-    grid_barrier(p.barrier, epoch);
-    // X = Y + Li^T T, with the column sums of squares of the new X (for the lazy normalisation)
-    const bool want_norm = (it & 1) && it != p.cholqr_at;
-    if (threadIdx.x < kMaxB) sG[threadIdx.x] = 0.0;
-    __syncthreads();
-    block_product(p.LiT, F, kUpper, p.T, nullptr, b, kc, sV, [&](int r, int j, double v) {
-      const double x = __ldcg(p.Y + (size_t)r * b + j) + v;
-      p.X[(size_t)r * b + j] = x;
-      if (want_norm) atomicAdd(&sG[j], x * x);
-    });
-    __syncthreads();
-    if (want_norm && threadIdx.x < b) atomicAdd(colsq + it * 32 + threadIdx.x, sG[threadIdx.x]);
-    scale_pending = want_norm;
-    scale_slot = it;
-    grid_barrier(p.barrier, epoch);
-    if (it == p.cholqr_at) {
-      // Cholesky-QR: G = X^T X, X <- X Lg^-T (every CTA factors the b x b Gram itself)
-      gram_accumulate(p.X, p.X, F, b, sG, G);
-      grid_barrier(p.barrier, epoch);
-      if (threadIdx.x == 0) {
-        for (int i = 0; i < b * b; ++i) sG[i] = __ldcg(G + i);
-        // Lg = chol(G) (lower) in sG; Linv = Lg^-1 in sL
-        for (int k = 0; k < b; ++k) {
-          double d = sG[k * b + k];
-          for (int m = 0; m < k; ++m) d -= sG[k * b + m] * sG[k * b + m];
-          d = sqrt(fmax(d, 1e-300));
-          sG[k * b + k] = d;
-          for (int i = k + 1; i < b; ++i) {
-            double s = sG[i * b + k];
-            for (int m = 0; m < k; ++m) s -= sG[i * b + m] * sG[k * b + m];
-            sG[i * b + k] = s / d;
-          }
-        }
-        for (int c = 0; c < b; ++c)
-          for (int r = 0; r < b; ++r) {
-            if (r < c) { sL[r * b + c] = 0.0; continue; }
-            double s = r == c ? 1.0 : 0.0;
-            for (int m = c; m < r; ++m) s -= sG[r * b + m] * sL[m * b + c];
-            sL[r * b + c] = s / sG[r * b + r];
-          }
-      }
-      __syncthreads();
-      for (int r0 = 0; r0 < F; r0 += rows_per_pass) {
-        const int r = r0 + blockIdx.x * kEigWarps + warp;
-        if (r >= F) continue;
-        const double x = lane < b ? __ldcg(p.X + (size_t)r * b + lane) : 0.0;
-        double out = 0.0;
-        for (int i = 0; i < b; ++i) {
-          const double xi = shfl_d(x, i);
-          if (lane < b && i <= lane) out = fma(xi, sL[lane * b + i], out);     // (X Lg^-T)[r][j] = sum_i x_i Linv[j][i]
-        }
-        if (lane < b) p.X[(size_t)r * b + lane] = out;
-      }
-      scale_pending = false;
-      grid_barrier(p.barrier, epoch);
-    }
-  }
-  // apply the pending column normalisation, then the Rayleigh-Ritz products
-  if (threadIdx.x < b) sS[threadIdx.x] = scale_pending ? rsqrt(__ldcg(colsq + scale_slot * 32 + threadIdx.x)) : 1.0;
-  __syncthreads();
-  if (scale_pending) {
-    for (int r0 = 0; r0 < F; r0 += rows_per_pass) {
-      const int r = r0 + blockIdx.x * kEigWarps + warp;
-      if (r < F && lane < b) p.X[(size_t)r * b + lane] = __ldcg(p.X + (size_t)r * b + lane) * sS[lane];
-    }
-    grid_barrier(p.barrier, epoch);
-  }
-  block_product(p.B, F, kFull, p.X, nullptr, b, kc, sV, [&](int r, int j, double v) { p.BX[(size_t)r * b + j] = v; });
-  block_product(p.Ct, F, kFull, p.X, nullptr, b, kc, sV, [&](int r, int j, double v) { p.CX[(size_t)r * b + j] = v; });
-  __syncthreads();
-  __threadfence_block();
-  // rows of BX / CX used below were written by this CTA's own warps (same row assignment)
-  gram_accumulate(p.X, p.BX, F, b, sG, Gb);
-  __syncthreads();
-  gram_accumulate(p.X, p.CX, F, b, sG, H);
-}
-
-__global__ void shift_matrix_kernel(const double* __restrict__ B, const double* __restrict__ Ct, double sigma,
-                                    double* __restrict__ K, double* __restrict__ K2, size_t n) {
-  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) {
-    const double v = sigma * B[i] - Ct[i];
-    K[i] = v;
-    if (K2) K2[i] = v;
-  }
-}
-
-}  // namespace
-}  // namespace dcg
-
-using namespace dcg;
-
-static int iter_kc(int F, int b) { return std::max(32, std::min((F + 31) / 32 * 32, (int)((160 * 1024 / 8) / b) / 32 * 32)); }
-
-extern "C" size_t dcg_eig_iterate_workspace_bytes(int F, int b, int n_iter) {
-  if (F < 1 || b < 1 || b > kMaxB || n_iter < 0) return 0;
-  // Z, T, Y, R (F x b each) + small block + barrier
-  return (size_t)4 * F * b * 8 + ((size_t)(n_iter + 1) * 32 + 3 * 1024) * 8 + 256;
-}
-
-// K = sigma B - Ct (F x F); the factorisation of K is the caller's (dcg_eig_chol_inv_f64).
-extern "C" int dcg_eig_shift_matrix_f64(const double* B, const double* Ct, int F, double sigma, double* K, double* K2,
-                                        void* stream) {
-  if (!B || !Ct || !K) return DCG_E_NULL;
-  if (F < 1) return DCG_E_SHAPE;
-  const size_t n = (size_t)F * F;
-  shift_matrix_kernel<<<(unsigned)ceil_div((int64_t)n, 256), 256, 0, (cudaStream_t)stream>>>(B, Ct, sigma, K, K2, n);
-  DCG_LAUNCH_CHECK();
-  return 0;
-}
-
-extern "C" int dcg_eig_iterate_f64(const double* B, const double* K, const double* Ct, const double* Li, const double* LiT,
-                                   int F, int b, int n_iter, int cholqr_at, double* X, double* BX, double* CX,
-                                   double* Gb, double* H, void* ws, size_t ws_bytes, void* stream) {
-  if (!B || !K || !Ct || !Li || !LiT || !X || !BX || !CX || !Gb || !H) return DCG_E_NULL;
-  if (F < 1 || b < 1 || b > kMaxB || n_iter < 0) return DCG_E_SHAPE;
-  if (!ws || ws_bytes < dcg_eig_iterate_workspace_bytes(F, b, n_iter)) return DCG_E_WORKSPACE;
-  cudaStream_t st = (cudaStream_t)stream;
-  double* w = (double*)ws;
-  IterParams p;
-  p.B = B; p.K = K; p.Ct = Ct; p.Li = Li; p.LiT = LiT; p.X = X;
-  p.Z = w; p.T = p.Z + (size_t)F * b; p.Y = p.T + (size_t)F * b; p.R = p.Y + (size_t)F * b;
-  p.small = p.R + (size_t)F * b;
-  const size_t n_small = (size_t)(n_iter + 1) * 32 + 3 * 1024;
-  p.barrier = (unsigned*)(p.small + n_small);
-  p.BX = BX; p.CX = CX;
-  p.F = F; p.b = b; p.n_iter = n_iter; p.cholqr_at = cholqr_at; p.kc = iter_kc(F, b);
-  DCG_CUDA_TRY(cudaMemsetAsync(p.small, 0, n_small * 8 + 64, st));
-  const size_t smem = (size_t)p.kc * b * 8;
-  DCG_CUDA_TRY(ensure_dynamic_smem((const void*)eig_iterate_kernel, smem));
-  int dev = 0, sms = 0;
-  DCG_CUDA_TRY(cudaGetDevice(&dev));
-  DCG_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  void* args[] = {(void*)&p};
-  DCG_CUDA_TRY(cudaLaunchCooperativeKernel((const void*)eig_iterate_kernel, dim3((unsigned)sms), dim3(kEigThreads), args, smem, st));
-  // Gb, H out of the small block
-  DCG_CUDA_TRY(cudaMemcpy2DAsync(Gb, (size_t)b * 8, p.small + (size_t)(n_iter + 1) * 32 + 1024, (size_t)b * 8, (size_t)b * 8, b,
-                                 cudaMemcpyDeviceToDevice, st));
-  DCG_CUDA_TRY(cudaMemcpy2DAsync(H, (size_t)b * 8, p.small + (size_t)(n_iter + 1) * 32 + 2048, (size_t)b * 8, (size_t)b * 8, b,
-                                 cudaMemcpyDeviceToDevice, st));
-  return 0;
-}
-
-// ======================================================================================================
-// Blocked Cholesky + triangular inverse (FP64), one persistent cooperative kernel
-// ======================================================================================================
-namespace dcg {
-namespace {
-
-constexpr int NB = 32;                    // block size = warp width
-constexpr int kPad = NB + 1;              // shared-memory row stride (doubles)
-
-struct CholParams {
-  double* A;          // F x F, row-major: in K (lower triangle used), out L in the lower triangle
-  int F;
-  double* Dinv;       // nb x 32 x 32: inverses of the diagonal blocks of L
-  double* Li;         // F x F: L^-1 (lower triangle written)
-  double* LiT;        // F x F: its transpose (upper triangle written)
-  double* status;     // [0] = 0 or 1 + index of the first non-positive pivot
-  unsigned* barrier;
-  int dbg;            // diagnostics (DCG_EIG_DBG)
-};
-
-// Cholesky of the 32 x 32 block whose row `lane` is a[0..lane] (in place: a becomes row `lane` of L),
-// then column `lane` of L^-1 in x[r], r >= lane (0 above).  `bad`: 1 + first non-positive pivot.
-__device__ __forceinline__ void warp_chol_inv(double (&a)[NB], double (&x)[NB], int lane, int& bad) {
-#pragma unroll
-  for (int k = 0; k < NB; ++k) {
-    double piv = shfl_d(a[k], k);
-    if (!(piv > 0.0)) { if (!bad) bad = k + 1; piv = 1.0; }
-    const double d = sqrt(piv);
-    const double l = a[k] / d;
-    a[k] = lane == k ? d : l;
-#pragma unroll
-    for (int c = k + 1; c < NB; ++c) a[c] = fma(-l, shfl_d(l, c), a[c]);
-  }
-  double dg = 1.0;
-#pragma unroll
-  for (int k = 0; k < NB; ++k) if (lane == k) dg = a[k];
-#pragma unroll
-  for (int r = 0; r < NB; ++r) {
-    double s = r == lane ? 1.0 : 0.0;
-#pragma unroll
-    for (int m = 0; m < r; ++m) s = fma(-shfl_d(a[m], r), x[m], s);
-    const double drr = shfl_d(dg, r);          // outside the conditional: every lane takes part in the shuffle
-    x[r] = r >= lane ? s / drr : 0.0;
-  }
-}
-
-// Factor the diagonal block whose (already updated) values sit in sO (rows 0..jb-1 valid), store L and Dinv.
-__device__ __noinline__ void factor_diag_block(const CholParams& p, int s, const double* sO, int lane) {
-  const int F = p.F, j0 = s * NB, jb = min(NB, F - j0);
-  double a[NB], x[NB];
-#pragma unroll
-  for (int c = 0; c < NB; ++c) {
-    double v = (lane < jb && c < jb && c <= lane) ? sO[lane * kPad + c] : 0.0;
-    if ((lane >= jb || c >= jb) && c == lane) v = 1.0;                 // identity padding of a partial block
-    a[c] = v;
-  }
-  int bad = 0;
-  warp_chol_inv(a, x, lane, bad);
-  if (bad && lane == 0 && p.status[0] == 0.0) p.status[0] = (double)(j0 + bad);
-#pragma unroll
-  for (int c = 0; c < NB; ++c)
-    if (lane < jb && c <= lane) p.A[(size_t)(j0 + lane) * F + j0 + c] = a[c];
-  double* D = p.Dinv + (size_t)s * NB * NB;
-#pragma unroll
-  for (int r = 0; r < NB; ++r) D[r * NB + lane] = x[r];               // column `lane` of the inverse
-}
-
-__global__ void __launch_bounds__(kEigThreads, 1) eig_chol_inv_kernel(const CholParams p) {
-  extern __shared__ __align__(16) double smem_c[];
-  const int F = p.F, nb = (F + NB - 1) / NB;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int gw = blockIdx.x * kEigWarps + warp, W = gridDim.x * kEigWarps;
-  double* sK = smem_c + (size_t)warp * 2 * NB * kPad;     // per warp: the k-panel block
-  double* sO = sK + NB * kPad;                            // per warp: the output tile
-  unsigned epoch = 0;
-  if (p.dbg == 1) return;
-  if (p.dbg == 2) { grid_barrier(p.barrier, epoch); return; }
-
-  // ---- first diagonal block
-  if (gw == 0) {
-    const int jb = min(NB, F);
-    for (int r = 0; r < NB; ++r)
-      sO[r * kPad + lane] = (r < jb && lane < jb) ? p.A[(size_t)r * F + lane] : 0.0;
-    __syncwarp();
-    factor_diag_block(p, 0, sO, lane);
-  }
-  if (p.dbg == 3) return;
-  if (p.dbg == 6) { __syncthreads(); return; }
-  grid_barrier(p.barrier, epoch);
-  if (p.dbg == 4) return;
-
-  for (int s = 0; s + 1 < nb; ++s) {
-    const int j0 = s * NB, t0 = j0 + NB;
-    // ---- panel: L[i, j0:j0+32] = A[i, j0:j0+32] Dinv_s^T for the rows below the diagonal block
-    {
-      const double* D = p.Dinv + (size_t)s * NB * NB;
-      double dr[NB];
-      bool loaded = false;
-      for (int i = t0 + gw; i < F; i += W) {
-        if (!loaded) {
-#pragma unroll
-          for (int m = 0; m < NB; ++m) dr[m] = __ldcg(D + lane * NB + m);       // row `lane` of Dinv (zero above the diagonal)
-          loaded = true;
-        }
-        const double am = __ldcg(p.A + (size_t)i * F + j0 + lane);
-        double out = 0.0;
-#pragma unroll
-        for (int m = 0; m < NB; ++m) out = fma(shfl_d(am, m), dr[m], out);
-        p.A[(size_t)i * F + j0 + lane] = out;
-      }
-    }
-    grid_barrier(p.barrier, epoch);
-    // ---- trailing update A[i][k] -= sum_m L[i][j0+m] L[k][j0+m] (lower triangle, 32 x 32 tiles); the warp
-    //      that owns the next diagonal tile factors it right away
-    {
-      const int nrem = nb - s - 1;
-      const int count = nrem * (nrem + 1) / 2;
-      for (int id = gw; id < count; id += (gw == 0 ? count : W - 1)) {
-        int ti = (int)((sqrt(8.0 * id + 1.0) - 1.0) * 0.5);
-        while ((ti + 1) * (ti + 2) / 2 <= id) ++ti;
-        while (ti * (ti + 1) / 2 > id) --ti;
-        const int tk = id - ti * (ti + 1) / 2;
-        const int ib = t0 + ti * NB, kb = t0 + tk * NB;
-        // stage the k-panel block and the output tile (coalesced rows)
-#pragma unroll 8
-        for (int c = 0; c < NB; ++c) {
-          const int kr = kb + c, ir = ib + c;
-          sK[c * kPad + lane] = kr < F ? __ldcg(p.A + (size_t)kr * F + j0 + lane) : 0.0;
-          sO[c * kPad + lane] = (ir < F && kb + lane < F) ? __ldcg(p.A + (size_t)ir * F + kb + lane) : 0.0;
-        }
-        __syncwarp();
-        double lrow[NB];
-        const int i = ib + lane;
-#pragma unroll
-        for (int m = 0; m < NB; ++m) lrow[m] = i < F ? __ldcg(p.A + (size_t)i * F + j0 + m) : 0.0;
-        for (int c = 0; c < NB; ++c) {
-          double dot = 0.0;
-#pragma unroll
-          for (int m = 0; m < NB; ++m) dot = fma(lrow[m], sK[c * kPad + m], dot);
-          sO[lane * kPad + c] -= dot;
-        }
-        __syncwarp();
-        if (id == 0) {
-          factor_diag_block(p, s + 1, sO, lane);             // next diagonal block: factor + invert + store
-        } else {
-#pragma unroll 8
-          for (int c = 0; c < NB; ++c) {
-            const int ir = ib + c;
-            if (ir < F && kb + lane < F) p.A[(size_t)ir * F + kb + lane] = sO[c * kPad + lane];
-          }
-        }
-        __syncwarp();
-      }
-    }
-    grid_barrier(p.barrier, epoch);
-  }
-
-  // ---- triangular inverse by independent block columns: Li_jj = Dinv_j, Li_ij = -Dinv_i sum_k L_ik Li_kj
-  double* sT = smem_c + (size_t)kEigWarps * 2 * NB * kPad;          // [8 warps][32][33] partial products
-  double* sD = sT + (size_t)kEigWarps * NB * kPad;                  // [32][33] Dinv_i
-  for (int j = blockIdx.x; j < nb; j += gridDim.x) {
-    // diagonal block
-    for (int e = threadIdx.x; e < NB * NB; e += kEigThreads) {
-      const int r = e / NB, c = e % NB;
-      const int gr = j * NB + r, gc = j * NB + c;
-      if (gr < F && gc < F) {
-        const double v = c <= r ? __ldcg(p.Dinv + (size_t)j * NB * NB + e) : 0.0;      // zeros above the diagonal
-        p.Li[(size_t)gr * F + gc] = v;
-        p.LiT[(size_t)gc * F + gr] = v;
-      }
-    }
-    __syncthreads();
-    for (int i = j + 1; i < nb; ++i) {
-      // partial T_w = sum over this warp's k of L_ik Li_kj
-      double acc[NB];
-#pragma unroll
-      for (int c = 0; c < NB; ++c) acc[c] = 0.0;
-      for (int k = j + warp; k < i; k += kEigWarps) {
-#pragma unroll 8
-        for (int m = 0; m < NB; ++m) {
-          const int gr = k * NB + m, gc = j * NB + lane;
-          sK[m * kPad + lane] = (gr < F && gc < F) ? __ldcg(p.Li + (size_t)gr * F + gc) : 0.0;   // Li_kj[m][lane]
-        }
-        __syncwarp();
-        const int gi = i * NB + lane;
-        double lrow[NB];
-#pragma unroll
-        for (int m = 0; m < NB; ++m) lrow[m] = (gi < F && k * NB + m < F) ? __ldcg(p.A + (size_t)gi * F + k * NB + m) : 0.0;
-#pragma unroll
-        for (int m = 0; m < NB; ++m) {
-          const double l = lrow[m];
-#pragma unroll
-          for (int c = 0; c < NB; ++c) acc[c] = fma(l, sK[m * kPad + c], acc[c]);
-        }
-        __syncwarp();
-      }
-#pragma unroll
-      for (int c = 0; c < NB; ++c) sT[((size_t)warp * NB + lane) * kPad + c] = acc[c];
-      for (int e = threadIdx.x; e < NB * NB; e += kEigThreads)
-        sD[(e / NB) * kPad + (e % NB)] = __ldcg(p.Dinv + (size_t)i * NB * NB + e);
-      __syncthreads();
-      // total T (in place in slice 0), then Li_ij = -Dinv_i T
-      for (int e = threadIdx.x; e < NB * NB; e += kEigThreads) {
-        const int r = e / NB, c = e % NB;
-        double t = 0.0;
-#pragma unroll
-        for (int w = 0; w < kEigWarps; ++w) t += sT[((size_t)w * NB + r) * kPad + c];
-        sT[(size_t)r * kPad + c] = t;          // slice 0, element (r, c): read above only by this thread for w = 0
-      }
-      __syncthreads();
-      for (int e = threadIdx.x; e < NB * NB; e += kEigThreads) {
-        const int r = e / NB, c = e % NB;
-        double v = 0.0;
-        for (int m = 0; m <= r; ++m) v = fma(sD[r * kPad + m], sT[(size_t)m * kPad + c], v);
-        const int gr = i * NB + r, gc = j * NB + c;
-        if (gr < F && gc < F) {
-          p.Li[(size_t)gr * F + gc] = -v;
-          p.LiT[(size_t)gc * F + gr] = -v;
-        }
-      }
-      __syncthreads();
-    }
-  }
-}
-
-}  // namespace
-}  // namespace dcg
-
-extern "C" size_t dcg_eig_chol_inv_workspace_bytes(int F) {
-  if (F < 1) return 0;
-  const size_t nb = (size_t)(F + 31) / 32;
-  return nb * 32 * 32 * 8 + 256;
-}
-
-extern "C" int dcg_eig_chol_inv_f64(double* K, int F, double* Li, double* LiT, double* status, void* ws, size_t ws_bytes,
-                                    void* stream) {
-  if (!K || !Li || !LiT || !status) return DCG_E_NULL;
-  if (F < 1) return DCG_E_SHAPE;
-  if (!ws || ws_bytes < dcg_eig_chol_inv_workspace_bytes(F)) return DCG_E_WORKSPACE;
-  cudaStream_t st = (cudaStream_t)stream;
-  const size_t nb = (size_t)(F + 31) / 32;
-  CholParams p;
-  p.A = K; p.F = F; p.Dinv = (double*)ws; p.Li = Li; p.LiT = LiT; p.status = status;
-  p.barrier = (unsigned*)((char*)ws + nb * 32 * 32 * 8);
-  p.dbg = getenv("DCG_EIG_DBG") ? atoi(getenv("DCG_EIG_DBG")) : 0;
-  DCG_CUDA_TRY(cudaMemsetAsync(p.barrier, 0, 64, st));
-  DCG_CUDA_TRY(cudaMemsetAsync(status, 0, sizeof(double), st));
-  const size_t smem = ((size_t)kEigWarps * 2 * NB * kPad + (size_t)kEigWarps * NB * kPad + (size_t)NB * kPad) * 8;
-  DCG_CUDA_TRY(ensure_dynamic_smem((const void*)eig_chol_inv_kernel, smem));
-  int dev = 0, sms = 0;
-  DCG_CUDA_TRY(cudaGetDevice(&dev));
-  DCG_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  void* args[] = {(void*)&p};
-  if (getenv("DCG_EIG_PLAIN_LAUNCH")) {
-    eig_chol_inv_kernel<<<(unsigned)sms, kEigThreads, smem, st>>>(p);
-    DCG_LAUNCH_CHECK();
-  } else {
-    DCG_CUDA_TRY(cudaLaunchCooperativeKernel((const void*)eig_chol_inv_kernel, dim3((unsigned)sms), dim3(kEigThreads), args, smem, st));
-  }
-  return 0;
-}
-
 
 // ---- inverses of the diagonal blocks of a lower-triangular matrix -----------------------------------------
 // The explicit inverse of the Cholesky factor of K (linalg._tri_inv_lower) is assembled bottom-up from the

@@ -94,8 +94,6 @@ def _shift_invert_topk(B: torch.Tensor, Ct: torch.Tensor, out: int, tol: float =
     them (in every pencil of the batch); returns None otherwise (flat spectrum, shift not found)
     and the caller goes dense."""
     batched = B.dim() == 3
-    if not batched and B.is_cuda and min(B.shape[-1], out + 8) <= 32 and os.environ.get("DCG_EIG_NATIVE", "0") == "1":
-        return _shift_invert_topk_native(B.contiguous(), Ct.contiguous(), out, tol, max_rounds)
     if not batched:
         B, Ct = B.unsqueeze(0), Ct.unsqueeze(0)
     nb, F = B.shape[0], B.shape[-1]
@@ -137,8 +135,6 @@ def _shift_invert_topk(B: torch.Tensor, Ct: torch.Tensor, out: int, tol: float =
         if host[-2] != 0 or host[0] != host[0]:
             return None
         worst = host[0]
-        if os.environ.get("DCG_EIG_DEBUG"):
-            print(f"[dcg eig] round {rnd}: {it} steps, worst relative residual {worst:.3e} (tol {tol:.1e})", flush=True)
         if worst <= tol:
             EIG_STATS["fast"] += nb
             EIG_STATS["last_iters"] = it
@@ -288,62 +284,6 @@ def _first_round(B, Ct, out, b):
     ent["Ct"].copy_(Ct)
     ent["graph"].replay()
     return ent["outs"]
-
-
-def _shift_invert_topk_native(B: torch.Tensor, Ct: torch.Tensor, out: int, tol: float = 1e-12, max_rounds: int = 10):
-    """The same iteration on the hand-written FP64 kernels of csrc/eig_dense.cu (one pencil): K = sigma B - Ct
-    and chol(K)^-1 in one persistent kernel (``ops.eig_factor``), all steps of a round + the Rayleigh-Ritz
-    products in another (``ops.eig_iterate``), the b x b pencil in ``dcg_gen_eig_small_f64`` -- no cuSOLVER /
-    cuBLAS kernel on the path.  Opt-in (DCG_EIG_NATIVE=1): correct to the same residual test, but at
-    F = 1000 the two kernels take 2.8 + 2.2 ms against 2.65 ms for the torch.linalg route (DESIGN.md 3.3)."""
-    from . import ops
-    F = B.shape[0]
-    b = min(F, out + 8)
-    nrm = torch.linalg.matrix_norm(Ct)
-    sigma = 1.05
-    fac = None
-    for _ in range(3):
-        K, Li, LiT, status = ops.eig_factor(B, Ct, sigma)
-        if float(status.item()) == 0.0:
-            fac = (K, Li, LiT)
-            break
-        sigma *= 2.0
-    if fac is None:
-        return None
-    X = _start_block(F, b, B.device).clone().contiguous()
-    it = 0
-    reshifted = False
-    for rnd in range(max_rounds):
-        n_it = 8 if rnd == 0 else 4
-        BX, CX, Gb, H = ops.eig_iterate(B, fac[0], Ct, fac[1], fac[2], X, n_it, 3 if rnd == 0 else -1)
-        it += n_it
-        theta, S, bad = ops.gen_eig_small(H.unsqueeze(0), Gb.unsqueeze(0))
-        theta, S = theta[0], S[0]
-        X = (X @ S).contiguous()
-        res = torch.linalg.norm(CX @ S[:, :out] - (BX @ S[:, :out]) * theta[None, :out], dim=0)
-        rel = res / (nrm * torch.linalg.norm(X[:, :out], dim=0))
-        host = torch.cat([rel.max().reshape(1), theta[0:1], theta[out - 1:out], theta[b - 1:b], bad.max().reshape(1)]).tolist()
-        if host[-1] != 0:
-            return None
-        if host[0] <= tol:
-            EIG_STATS["fast"] += 1
-            EIG_STATS["last_iters"] = it
-            return theta[:out], X[:, :out]
-        if not reshifted:
-            reshifted = True
-            th0, tho, thb = host[1], host[2], host[3]
-            rate = (sigma - tho) / max(sigma - thb, 1e-300)
-            if rate > 0.25:
-                for mult in (0.05, 0.2, 0.8):
-                    s2 = min(sigma, th0 + mult * max(th0 - thb, 1e-12) + 1e-9 * max(1.0, abs(th0)))
-                    K, Li, LiT, status = ops.eig_factor(B, Ct, s2)
-                    if float(status.item()) == 0.0:
-                        fac, sigma = (K, Li, LiT), s2
-                        break
-            rate = (sigma - tho) / max(sigma - thb, 1e-300)
-            if rate >= 1.0 or math.log(tol) / math.log(max(rate, 1e-300)) > 4 * max_rounds:
-                return None
-    return None
 
 
 def _cholesky_eigh(C0: torch.Tensor, Ct: torch.Tensor, reg: float, out: int):

@@ -831,49 +831,3 @@ def tri_inv_blocks_(L: torch.Tensor, out: torch.Tensor, nblk: int, bs: int) -> t
           L.stride(1), L.stride(2), L.stride(0), out.stride(1), out.stride(2), out.stride(0), _stream(L.device))
     _count(1)
     return out
-
-
-def eig_factor(B: torch.Tensor, Ct: torch.Tensor, sigma: float):
-    """K = sigma B - Ct and the explicit inverse of its Cholesky factor, on the hand-written FP64 kernels
-    (csrc/eig_dense.cu).  Returns (K, Li, LiT, status): K as formed (F x F), Li = chol(K)^-1 (lower),
-    LiT = Li^T, status (1,) device FP64 = 0 or 1 + the first non-positive pivot."""
-    _need_cuda("B", B, torch.float64)
-    _need_cuda("Ct", Ct, torch.float64)
-    F = B.shape[0]
-    if B.shape != (F, F) or Ct.shape != (F, F) or not B.is_contiguous() or not Ct.is_contiguous():
-        raise ValueError("B and Ct must be contiguous (F, F)")
-    lib = _lib.load()
-    dev = B.device
-    K = torch.empty_like(B)
-    L = torch.empty_like(B)                                  # the factorisation overwrites its input
-    _call(dev, "dcg_eig_shift_matrix_f64", B.data_ptr(), Ct.data_ptr(), F, float(sigma), K.data_ptr(), L.data_ptr(),
-          _stream(dev))
-    Li = torch.empty_like(B)                                 # only the lower (LiT: upper) triangle is written
-    LiT = torch.empty_like(B)
-    status = torch.empty(1, dtype=torch.float64, device=dev)
-    ws = _ws(lib.dcg_eig_chol_inv_workspace_bytes(F), dev)
-    _call(dev, "dcg_eig_chol_inv_f64", L.data_ptr(), F, Li.data_ptr(), LiT.data_ptr(), status.data_ptr(),
-          ws.data_ptr(), ws.numel(), _stream(dev))
-    _count(2)
-    return K, Li, LiT, status
-
-
-def eig_iterate(B, K, Ct, Li, LiT, X: torch.Tensor, n_iter: int, cholqr_at: int = -1):
-    """``n_iter`` steps of X <- K^-1 B X on the (F, b) block X IN PLACE (one persistent kernel), then the
-    Rayleigh-Ritz products.  Returns (BX, CX, Gb, H)."""
-    _need_cuda("X", X, torch.float64)
-    F, b = X.shape
-    if not X.is_contiguous() or b > 32:
-        raise ValueError("X must be contiguous (F, b) with b <= 32")
-    lib = _lib.load()
-    dev = X.device
-    BX = torch.empty_like(X)
-    CX = torch.empty_like(X)
-    Gb = torch.empty((b, b), dtype=torch.float64, device=dev)
-    H = torch.empty((b, b), dtype=torch.float64, device=dev)
-    ws = _ws(lib.dcg_eig_iterate_workspace_bytes(F, b, n_iter), dev)
-    _call(dev, "dcg_eig_iterate_f64", B.data_ptr(), K.data_ptr(), Ct.data_ptr(), Li.data_ptr(), LiT.data_ptr(), F, b,
-          int(n_iter), int(cholqr_at), X.data_ptr(), BX.data_ptr(), CX.data_ptr(), Gb.data_ptr(), H.data_ptr(),
-          ws.data_ptr(), ws.numel(), _stream(dev))
-    _count(1)
-    return BX, CX, Gb, H

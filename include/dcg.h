@@ -277,20 +277,6 @@ int dcg_ticaloss_f64(const double* sums, int d, double reg, int n_eig, double* r
 int dcg_gen_eig_small_f64(const double* H, const double* G, int b, int batch,
                           double* theta, double* S, double* status, void* stream);
 
-/* ---- E1: F x F generalised eigenproblem, leading eigenpairs (FP64, one device) ----------------------
- * Replaces mlcolvar `cholesky_eigh` inside `TICA.compute` (cv_calculator.py:2257-2261, 2350-2354,
- * 2374-2378) for the leading eigenpairs by shift-and-invert subspace iteration (csrc/eig_dense.cu,
- * linalg.py).  All matrices row-major FP64.
- *   dcg_eig_shift_matrix_f64  K = sigma B - Ct, written to K and (if not NULL) to K2 -- the copy the
- *                             factorisation may overwrite.
- *   dcg_eig_chol_inv_f64      Li = chol(K)^-1 (only its lower triangle is written) and LiT = Li^T (upper
- *                             triangle); K is overwritten with its Cholesky factor; status[0] (device) = 0,
- *                             or 1 + the first pivot that is not positive.  ws: dcg_eig_chol_inv_workspace_bytes(F).
- *   dcg_eig_iterate_f64       n_iter steps of X <- K^-1 B X on the F x b block X (b <= 32; K^-1 applied as
- *                             Li^T Li with one step of iterative refinement; columns re-normalised every
- *                             other step, one Cholesky-QR after step `cholqr_at`, -1 for none), then
- *                             BX = B X, CX = Ct X (F x b) and the b x b Rayleigh-Ritz matrices
- *                             Gb = X^T B X, H = X^T Ct X.  One persistent cooperative kernel.          */
 /* Inverses of the `nblk` diagonal blocks (bs x bs, bs <= 128) of `batch` lower-triangular matrices, written to
  * the same blocks of `out`; element (i, j) of matrix m at m * sbatch + i * srow + j * scol (any layout).  One CTA
  * per block, forward substitution, no synchronisation (part of the explicit inverse of chol(K) in the
@@ -298,15 +284,6 @@ int dcg_gen_eig_small_f64(const double* H, const double* G, int b, int batch,
 int dcg_tri_inv_blocks_f64(const double* L, double* out, int batch, int nblk, int bs,
                            int64_t srow, int64_t scol, int64_t sbatch,
                            int64_t orow, int64_t ocol, int64_t obatch, void* stream);
-int dcg_eig_shift_matrix_f64(const double* B, const double* Ct, int F, double sigma, double* K, double* K2,
-                             void* stream);
-size_t dcg_eig_chol_inv_workspace_bytes(int F);
-int dcg_eig_chol_inv_f64(double* K, int F, double* Li, double* LiT, double* status, void* ws, size_t ws_bytes,
-                         void* stream);
-size_t dcg_eig_iterate_workspace_bytes(int F, int b, int n_iter);
-int dcg_eig_iterate_f64(const double* B, const double* K, const double* Ct, const double* Li, const double* LiT,
-                        int F, int b, int n_iter, int cholqr_at, double* X, double* BX, double* CX,
-                        double* Gb, double* H, void* ws, size_t ws_bytes, void* stream);
 
 /* ---- N1: dispersion sums for the clustering scores -------------------------------------------------
  * For sklearn's calinski_harabasz_score / davies_bouldin_score as called at

@@ -1474,37 +1474,3 @@ def test_normalisation_modes_through_the_fused_kernels(dev, tmp_path, mode, engi
     Pn_ref, _, _ = f64.project_normalized(Xd, mean, rng, V_ref)
     sgn = torch.sign((torch.from_numpy(calc.cv).to(dev).double() * V_ref).sum(0, keepdim=True))
     assert (P.double() * sgn - Pn_ref).abs().max().item() < 1e-4 or engine != "auto"
-
-
-# ------------------------------------------------------------------------------------------------
-# E1: hand-written FP64 eigen-stage kernels (opt-in path)
-# ------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("F", [1000, 333, 50])
-def test_native_eigen_kernels_match_torch_linalg(dev, monkeypatch, F):
-    """csrc/eig_dense.cu: blocked Cholesky + triangular inverse and the persistent shift-and-invert
-    iteration against torch.linalg, then the whole solve (DCG_EIG_NATIVE=1) against the dense
-    Cholesky -> eigh route of the reference."""
-    from deep_cartograph_b200 import linalg, ops
-    from oracle import float64_device as f64
-    n, lag, out = 60_000, 10, 4
-    X = _cuda(synth_features(n, F, seed=F), dev)
-    st = ops.column_stats(X)
-    mean, rng = st["mean"].float(), torch.sqrt(st["m2"] / (n - 1)).float()
-    ref = f64.lagged_sums(X, lag, mean, rng)
-    M = ref["M"]
-    mu, nu = ref["a"] / M, ref["b"] / M
-    C0 = ref["S0"] / M - torch.outer(mu, mu); C0 = 0.5 * (C0 + C0.T)
-    Ct = ref["St"] / M - torch.outer(mu, nu); Ct = (0.5 * (Ct + Ct.T)).contiguous()
-    B = (C0 + 1e-6 * torch.eye(F, dtype=torch.float64, device=dev)).contiguous()
-    K, Li, LiT, status = ops.eig_factor(B, Ct, 1.05)
-    assert status.item() == 0.0
-    Liref = torch.linalg.inv(torch.linalg.cholesky(K))
-    scale = Liref.abs().max()
-    assert ((torch.tril(Li) - Liref).abs().max() / scale).item() < 1e-11
-    assert ((torch.triu(LiT) - Liref.T).abs().max() / scale).item() < 1e-11
-    monkeypatch.setenv("DCG_EIG_NATIVE", "1")
-    ev, V = linalg.tica_from_sums(ref["S0"], ref["St"], ref["a"], ref["b"], M, out)
-    monkeypatch.delenv("DCG_EIG_NATIVE")
-    ev_ref, V_ref = f64.tica_from_sums(ref["S0"], ref["St"], ref["a"], ref["b"], M, out)
-    assert ((ev - ev_ref).abs() / ev_ref.abs()).max().item() < 1e-9
-    assert f64.eigvec_error(V, V_ref) < 1e-7
