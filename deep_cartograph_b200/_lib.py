@@ -25,6 +25,8 @@ COV_ENGINES = {"simt_f32": COV_SIMT_F32, "tc_3xtf32": COV_TC_3XTF32, "tc_1xtf32"
 
 LINKAGE_METHODS = {"single": 0, "complete": 1, "average": 2, "ward": 3}   # DCG_LINK_* (dcg.h)
 HDBSCAN_MAX_MIN_SAMPLES = 64                                              # DCG_HDBSCAN_MAX_MIN_SAMPLES (dcg.h)
+SILHOUETTE_MAX_SLOTS = 384                                                # DCG_SILHOUETTE_MAX_SLOTS (dcg.h)
+SILHOUETTE_MAX_LABELINGS = 32                                             # DCG_SILHOUETTE_MAX_LABELINGS (dcg.h)
 
 _SIGNATURES = {
     # name: (restype, [argtypes])
@@ -72,6 +74,8 @@ _SIGNATURES = {
     "dcg_gen_eig_small_f64": (_c_int, [_p, _p, _c_int, _c_int, _p, _p, _p, _p]),
     "dcg_tri_inv_blocks_f64": (_c_int, [_p, _p, _c_int, _c_int, _c_int, _c_i64, _c_i64, _c_i64, _c_i64, _c_i64, _c_i64, _p]),
     "dcg_cluster_dispersion": (_c_int, [_p, _c_i64, _c_int, _c_i64, _c_int, _p, _p, _c_int, _p, _p, _p]),
+    "dcg_silhouette_workspace_bytes": (_c_sz, [_c_i64, _c_int, _c_int]),
+    "dcg_silhouette_f64": (_c_int, [_p, _c_i64, _c_int, _c_i64, _p, _c_int, _p, _p, _c_int, _p, _p, _p, _c_sz, _p]),
     "dcg_linkage_workspace_bytes": (_c_sz, [_c_i64, _c_int, _c_int]),
     "dcg_linkage_f64": (_c_int, [_p, _c_i64, _c_int, _c_i64, _c_int, _p, _p, _c_sz, _p]),
     "dcg_hdbscan_workspace_bytes": (_c_sz, [_c_i64, _c_int, _c_int]),

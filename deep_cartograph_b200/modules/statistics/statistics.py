@@ -302,41 +302,27 @@ def cluster_scores(features, labels, centers=None) -> Dict[str, float]:
     return {"calinski_harabasz": float(ch), "davies_bouldin": db}
 
 
-def silhouette(features, labels, sample_size: Optional[int] = None, seed: int = 0, chunk: int = 2048) -> float:
-    """Mean silhouette coefficient (sklearn ``silhouette_score``, Euclidean; reference statistics.py:75)
-    on the device in FP64: for every frame i, a_i = mean distance to the other members of its cluster,
+def silhouettes(features, labelings, sample_size: Optional[int] = None, seed: int = 0) -> List[float]:
+    """Mean silhouette coefficient (sklearn ``silhouette_score``, Euclidean; reference statistics.py:75) of
+    every labeling of the same frames, exact in FP64 on the device, all labelings in one pass over the frame
+    pairs (``ops.silhouette``): for every frame i, a_i = mean distance to the other members of its cluster,
     b_i = the smallest mean distance to the members of another cluster, s_i = (b_i - a_i) / max(a_i, b_i)
-    (0 for singleton clusters).  O(N^2 d): ``sample_size`` evaluates it on a uniform random subsample
-    of that many frames against each other -- sklearn's own ``sample_size`` estimator."""
-    Y = _to_device(features).to(torch.float64)
-    lab = torch.as_tensor(np.asarray(labels), device=Y.device).long()
+    (0 for singleton clusters and for a_i = b_i = 0).  O(N^2 d) work, O(N (d + L)) memory.  ``sample_size``
+    evaluates it on a uniform random subsample of that many frames against each other -- sklearn's own
+    ``sample_size`` estimator, the same subsample (``RandomState(seed).permutation(n)[:sample_size]``) for
+    every labeling."""
+    Y = _to_device(features)
+    labs = torch.stack([torch.as_tensor(np.asarray(lab), device=Y.device).long() for lab in labelings])
     n = Y.shape[0]
     if sample_size is not None and sample_size < n:
         idx = torch.from_numpy(np.random.RandomState(seed).permutation(n)[:sample_size]).to(Y.device)
-        Y, lab = Y[idx], lab[idx]
-        n = sample_size
-    ids, inv = torch.unique(lab, return_inverse=True)
-    k = ids.numel()
-    if not 2 <= k <= n - 1:
-        raise ValueError("Number of labels is %d. Valid values are 2 to n_samples - 1 (inclusive)" % k)
-    onehot = torch.zeros((n, k), dtype=torch.float64, device=Y.device)
-    onehot[torch.arange(n, device=Y.device), inv] = 1.0
-    cnt = onehot.sum(dim=0)
-    total = torch.zeros((), dtype=torch.float64, device=Y.device)
-    for s0 in range(0, n, chunk):
-        e0 = min(n, s0 + chunk)
-        Dc = torch.cdist(Y[s0:e0], Y) @ onehot                          # (chunk, k): summed distances to every cluster
-        own = inv[s0:e0]
-        rows = torch.arange(e0 - s0, device=Y.device)
-        n_own = cnt[own]
-        a = Dc[rows, own] / (n_own - 1).clamp(min=1.0)
-        Dm = Dc / cnt[None, :]
-        Dm[rows, own] = float("inf")
-        b = Dm.min(dim=1).values
-        sil = (b - a) / torch.maximum(a, b)
-        sil = torch.where(n_own > 1, sil, torch.zeros_like(sil))
-        total += torch.nan_to_num(sil).sum()
-    return float((total / n).item())
+        Y, labs = Y[idx], labs[:, idx]
+    return ops.silhouette(Y, labs).tolist()
+
+
+def silhouette(features, labels, sample_size: Optional[int] = None, seed: int = 0) -> float:
+    """Mean silhouette coefficient of one labeling (``silhouettes``)."""
+    return silhouettes(features, [labels], sample_size, seed)[0]
 
 
 def optimize_clustering(features, settings: Dict):
@@ -345,9 +331,11 @@ def optimize_clustering(features, settings: Dict):
     refitting per k gives): every k of ``search_interval`` is clustered and scored
     with Calinski-Harabasz, Davies-Bouldin and the mean silhouette; each score is min-max normalised over
     the interval and the best k maximises (CH - DB + silhouette) / 3.  Like the reference it mutates
-    ``settings['num_clusters']`` and ignores ``opt_num_clusters``.  The silhouette is exact up to
-    ``settings['silhouette_max_samples']`` frames (default 50000, O(N^2) on the device); beyond that it is
-    sklearn's ``sample_size`` estimator on that many frames (seed 0) and a warning says so.
+    ``settings['num_clusters']`` and ignores ``opt_num_clusters``.  Every k is clustered first, then the
+    silhouettes of all k are computed together in one pass over the frame pairs (``silhouettes``).  The
+    silhouette is exact up to ``settings['silhouette_max_samples']`` frames (default 50000; None: every frame,
+    at any N); beyond that it is sklearn's ``sample_size`` estimator on that many frames (seed 0, the same
+    subsample for every k) and a warning says so.
     HDBSCAN (with ``backend.hdbscan_on_device``) takes no number of clusters: it runs once, unscored."""
     algorithm = settings.get("algorithm", "kmeans")
     tree = None
@@ -365,13 +353,13 @@ def optimize_clustering(features, settings: Dict):
     lo, hi = settings.get("search_interval", [2, 15])
     ks = list(range(lo, hi + 1))
     feats = np.asarray(features)
-    max_sil = int(settings.get("silhouette_max_samples", 50000))
+    max_sil = settings.get("silhouette_max_samples", 50000)
     sample = None
-    if feats.shape[0] > max_sil:
-        sample = max_sil
-        logger.warning(f"Silhouette score estimated on a random subsample of {max_sil} of {feats.shape[0]} frames "
+    if max_sil is not None and feats.shape[0] > int(max_sil):
+        sample = int(max_sil)
+        logger.warning(f"Silhouette score estimated on a random subsample of {sample} of {feats.shape[0]} frames "
                        "(scikit-learn's sample_size estimator); the reference evaluates all pairs")
-    ch, db, sil, results = [], [], [], []
+    ch, db, results = [], [], []
     for k in ks:
         settings["num_clusters"] = k
         if tree is None:
@@ -382,11 +370,11 @@ def optimize_clustering(features, settings: Dict):
         sc = cluster_scores(feats, labels)
         ch.append(sc["calinski_harabasz"])
         db.append(sc["davies_bouldin"])
-        sil.append(silhouette(feats, labels, sample_size=sample))
-        logger.debug(f"Calinski-Harabasz score: {round(ch[-1], 3)}")
-        logger.debug(f"Davies-Bouldin score: {round(db[-1], 3)}")
-        logger.debug(f"Average silhouette score: {round(sil[-1], 3)}")
         results.append((labels, centroids))
+    sil = silhouettes(feats, [labels for labels, _ in results], sample_size=sample)
+    for k, c, b, s in zip(ks, ch, db, sil):
+        logger.debug(f"k = {k}: Calinski-Harabasz score: {round(c, 3)}, Davies-Bouldin score: {round(b, 3)}, "
+                     f"average silhouette score: {round(s, 3)}")
 
     def norm(v):
         v = np.asarray(v, dtype=np.float64)

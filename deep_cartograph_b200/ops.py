@@ -648,6 +648,87 @@ def cluster_dispersion(Y: torch.Tensor, labels: torch.Tensor, means: torch.Tenso
     return ssq, sdist
 
 
+def _silhouette_groups(ks, max_slots: int = _lib.SILHOUETTE_MAX_SLOTS,
+                       max_labelings: int = _lib.SILHOUETTE_MAX_LABELINGS):
+    """Consecutive groups of labelings (lists of indices) whose cluster counts ``ks`` add up to at most
+    ``max_slots`` with at most ``max_labelings`` labelings each: one kernel pass per group."""
+    groups, cur, slots = [], [], 0
+    for i, k in enumerate(ks):
+        if cur and (slots + k > max_slots or len(cur) == max_labelings):
+            groups.append(cur)
+            cur, slots = [], 0
+        cur.append(i)
+        slots += k
+    if cur:
+        groups.append(cur)
+    return groups
+
+
+def silhouette(Y: torch.Tensor, labelings, return_samples: bool = False):
+    """Exact mean silhouette coefficient (scikit-learn's ``silhouette_score``, Euclidean) of every labeling of
+    the frames ``Y`` (n x d CUDA tensor, float32 widened exactly, or float64; finite), all labelings in one pass
+    over the frame pairs (csrc/silhouette.cu; see dcg.h, N1).  ``labelings``: one labeling (n,) or several
+    (L, n), or a sequence of them; any integer values, encoded 0..k-1 as scikit-learn's LabelEncoder does, with
+    2 <= k <= n - 1.  Returns the L means as a float64 tensor, and with ``return_samples`` also the (L, n) per-frame
+    values (``silhouette_samples``).  Labelings whose clusters together exceed the kernel's 384 slots (or
+    more than 32 labelings) are scored in several passes; a labeling's result does not depend on the grouping."""
+    Y = _nearest_rows("Y", Y)
+    n, d = Y.shape
+    if isinstance(labelings, torch.Tensor) and labelings.dim() == 1:
+        labelings = [labelings]
+    labs = [torch.as_tensor(lab, device=Y.device) for lab in labelings]
+    if not labs:
+        raise ValueError("labelings must hold at least one labeling")
+    if d > 2048:
+        raise ValueError(f"the silhouette kernel takes at most 2048 features, got {d}")
+    codes, sizes, ks = [], [], []
+    for lab in labs:
+        if lab.dim() != 1 or lab.shape[0] != n:
+            raise ValueError(f"every labeling must have one label per frame ({n}), got shape {tuple(lab.shape)}")
+        if lab.dtype.is_floating_point or lab.dtype == torch.bool:
+            raise TypeError(f"labels must be integers, got {lab.dtype}")
+        _, inv = torch.unique(lab, return_inverse=True)
+        k = int(inv.max().item()) + 1 if n > 0 else 0
+        if not 2 <= k <= n - 1:
+            raise ValueError("Number of labels is %d. Valid values are 2 to n_samples - 1 (inclusive)" % k)
+        if k > _lib.SILHOUETTE_MAX_SLOTS:
+            raise ValueError(f"the silhouette kernel scores at most {_lib.SILHOUETTE_MAX_SLOTS} clusters per labeling, "
+                             f"got {k}")
+        codes.append(inv.to(torch.int32))
+        sizes.append(torch.bincount(inv, minlength=k).to(torch.int32))
+        ks.append(k)
+    dev = Y.device
+    groups = _silhouette_groups(ks)
+    lib = _lib.load()
+    nbytes = max(int(lib.dcg_silhouette_workspace_bytes(n, len(g), sum(ks[i] for i in g))) for g in groups)
+    if nbytes == 0:
+        raise ValueError(f"silhouette of {n} frames: shape out of range")
+    L = len(labs)
+    need = nbytes + 4 * n * L + (16 * n * L if return_samples else 0)
+    free, _ = torch.cuda.mem_get_info(dev)
+    if need > free:
+        raise MemoryError(f"silhouette of {n} frames and {L} labelings needs {need} bytes of device memory; "
+                          f"{free} bytes are free")
+    ws = _ws(nbytes, dev)
+    scores = torch.empty(L, dtype=torch.float64, device=dev)
+    samples = torch.empty((L, n), dtype=torch.float64, device=dev) if return_samples else None
+    for g in groups:
+        lab_g = torch.stack([codes[i] for i in g]).contiguous()
+        kg = [ks[i] for i in g]
+        offsets = torch.tensor([sum(kg[:j]) for j in range(len(kg) + 1)], dtype=torch.int32, device=dev)
+        sizes_g = torch.cat([sizes[i] for i in g]).contiguous()
+        out = torch.empty(len(g), dtype=torch.float64, device=dev)
+        smp = torch.empty((len(g), n), dtype=torch.float64, device=dev) if return_samples else None
+        _call(dev, "dcg_silhouette_f64", Y.data_ptr(), n, d, d, lab_g.data_ptr(), len(g), offsets.data_ptr(),
+              sizes_g.data_ptr(), sum(kg), out.data_ptr(), _ptr(smp), ws.data_ptr(), ws.numel(), _stream(dev))
+        _count(3)                  # prep, pass, reduce
+        idx = torch.tensor(g, device=dev)
+        scores[idx] = out
+        if return_samples:
+            samples[idx] = smp
+    return (scores, samples) if return_samples else scores
+
+
 # ---- N2: agglomerative clustering tree ------------------------------------------------------------------
 def linkage(Y: torch.Tensor, method: str = "complete", return_phases: bool = False):
     """Merge tree of the frames ``Y`` (n x d CUDA tensor, float32 or float64) for ``method`` in

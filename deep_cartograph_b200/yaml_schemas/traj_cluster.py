@@ -39,4 +39,7 @@ class TrajClusterSchema(BaseModel):
     cluster_selection_epsilon: float = 0
     cluster_selection_method: Literal["eom", "leaf"] = "eom"
     figures: Dict = {}
+    # frames above which optimize_clustering estimates the silhouette on a random subsample of this many frames
+    # (scikit-learn's sample_size estimator, seed 0); null: the exact score over every frame pair, at any N
+    silhouette_max_samples: Optional[int] = 50000
     backend: Backend = Backend()

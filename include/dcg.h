@@ -293,6 +293,35 @@ int dcg_tri_inv_blocks_f64(const double* L, double* out, int batch, int nblk, in
 int dcg_cluster_dispersion(const void* Y, int64_t n, int d, int64_t ld, int dtype_bytes, const int* labels,
                            const double* means, int k, double* ssq, double* sdist, void* stream);
 
+/* ---- N1: exact silhouette of L labelings in one pass over all frame pairs ------------------------------
+ * For sklearn's silhouette_score(metric="euclidean") as called at modules/statistics/statistics.py:75, for
+ * L labelings of the same n frames Y (n x d FP64, row stride ld) at once (csrc/silhouette.cu).  Per labeling
+ * l, with its labels encoded 0..k_l - 1 (as LabelEncoder does):
+ *   a_i = (sum of d(i, j) over i's own cluster) / (n_own - 1),
+ *   b_i = min over the other clusters c of (sum of d(i, j) over c) / |c|,
+ *   s_i = (b_i - a_i) / max(a_i, b_i), NaN -> 0 (singletons; a = b = 0), scores[l] = mean of s_i.
+ * d(i, j) = sqrt(sum_f (y_i[f] - y_j[f])^2), features ascending, a rounded subtract, multiply and add per term,
+ * then one sqrt (pdist's arithmetic, as dcg_linkage_f64 and dcg_nearest_frames_f64).  Each distance is computed
+ * once and feeds every labeling; each cluster sum of m distances is within m u / (1 - m u) of exact (u = 2^-53).
+ * A labeling's results are bitwise the same whether it is scored alone or with others, and from run to run
+ * (fixed-order sums, no floating-point atomics).
+ * Inputs (device): labels L x n int32 (labeling l at labels + l n); offsets L + 1 int32, labeling l owns slots
+ * offsets[l] .. offsets[l+1] - 1, offsets[0] = 0, offsets[L] = K = sum_l k_l; sizes K int32, the member count
+ * of every slot.  Outputs: scores (L doubles); samples (L x n doubles, s_i of labeling l at samples + l n; may
+ * be NULL).  A label outside 0..k_l - 1 touches no slot: that labeling's score is NaN, as is s_i of its frame.
+ * Limits: every slot has one FP64 accumulator per row of a CTA in shared memory, so K <= 384
+ * (DCG_SILHOUETTE_MAX_SLOTS: 192 KB of the 227 KB a CTA may use), L <= 32, d <= 2048; callers split larger
+ * sets of labelings into groups.  Memory is O(n (d + L)): the workspace holds n (4 + 2 L) bytes of label
+ * codes and masks and 8 L doubles per 64 frames, no n x n or chunk x n buffer.  O(n^2 (d + L)) work.
+ * Errors: DCG_E_SHAPE for n < 3, n > INT_MAX, d < 1, d > 2048, ld < d, L < 1, L > 32, K < 2 L or K > 384;
+ * DCG_E_NULL (samples may be NULL); DCG_E_WORKSPACE.  The workspace query returns 0 for an invalid shape.    */
+#define DCG_SILHOUETTE_MAX_SLOTS     384
+#define DCG_SILHOUETTE_MAX_LABELINGS 32
+size_t dcg_silhouette_workspace_bytes(int64_t n, int L, int K);
+int dcg_silhouette_f64(const double* Y, int64_t n, int d, int64_t ld, const int32_t* labels, int L,
+                       const int32_t* offsets, const int32_t* sizes, int K, double* scores, double* samples,
+                       void* ws, size_t ws_bytes, void* stream);
+
 /* ---- N2: agglomerative clustering tree ----------------------------------------------------------------
  * Replaces sklearn AgglomerativeClustering(n_clusters, linkage).fit_predict as called from
  * `hierarchical_clustering` (modules/statistics/statistics.py:285): the full merge tree of the n frames of
